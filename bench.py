@@ -303,6 +303,52 @@ def timed_device_steps(I, plumb, method, steps, warmup, sampler=None, chunks=1):
             "step_ms_median": plumb.max(float(np.median(step_ms))), "step_ms_best": plumb.max(float(np.min(step_ms)))}
 
 
+DUMP_ROWS = 1 << 16        # CSR rows sampled by --dump-outputs
+DUMP_SEED = 0
+DUMP_BYTES = 64 << 20      # all files together, .npy headers included
+DUMP_CHUNK = 1 << 22       # entries per pass of the whole-result sums (bounds their temporaries)
+
+
+def dump_outputs(I, out_dir):
+    """Write what the last device step computed, as the caller of interpolate() would receive it, under out_dir.
+
+    The whole CSR of the default workload is ~2.4 GB, so a fixed seeded sample of DUMP_ROWS rows is written: their ids
+    (rows), entry counts (row_nnz), element ids (indices), weights (data) and neumann weights (neumann).  totals holds
+    sums over the whole result, so that a difference outside the sample still shows: [n_rows, n_cols, nnz, NaN count,
+    nansum(data), nansum(|data|), nansum(data * (indices + 1)), nansum(neumann)], the entry sums taken DUMP_CHUNK
+    entries at a time.  Every file is float64, and all of them together take at most DUMP_BYTES."""
+    ctx, g = I._ctx, I.grid
+    n_rows, n_cols = int(g.n_points), int(g.n_elems)
+    indptr = np.empty(n_rows + 1, dtype=np.int32)
+    neumann = np.empty(n_rows, dtype=np.float64)
+    ctx.interpolate_fetch(indptr, None, None, neumann)
+    nnz = int(indptr[-1])
+    indices = np.empty(nnz, dtype=np.int32)
+    data = np.empty(nnz, dtype=np.float64)
+    ctx.interpolate_fetch(None, indices, data, None)
+    perm = np.random.default_rng(DUMP_SEED).permutation(n_rows)
+    k = min(n_rows, DUMP_ROWS)
+    fixed = 8 * 8 + 6 * 256                 # totals, and six .npy headers (128 bytes each for 1-D arrays)
+    while True:
+        rows = np.sort(perm[:k])
+        counts = (indptr[rows + 1] - indptr[rows]).astype(np.int64)
+        if 16 * int(counts.sum()) + 24 * k + fixed <= DUMP_BYTES or k == 1:
+            break
+        k //= 2
+    starts = indptr[rows].astype(np.int64)
+    at = np.repeat(starts - (np.cumsum(counts) - counts), counts) + np.arange(int(counts.sum()))
+    sums = np.zeros(4)                      # NaN count, nansum(data), nansum(|data|), nansum(data * (indices + 1))
+    for b in range(0, nnz, DUMP_CHUNK):
+        d, ix = data[b:b + DUMP_CHUNK], indices[b:b + DUMP_CHUNK]
+        sums += [np.isnan(d).sum(), np.nansum(d), np.nansum(np.abs(d)), np.nansum(d * (ix + 1.0))]
+    totals = [n_rows, n_cols, nnz, *sums, np.nansum(neumann)]
+    out = {"rows": rows, "row_nnz": counts, "indices": indices[at], "data": data[at], "neumann": neumann[rows], "totals": totals}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
+    log(f"dumped {k} of {n_rows} rows ({int(counts.sum())} of {nnz} entries) to {out_dir}")
+
+
 def timed_e2e_steps(I, plumb, method, steps, warmup):
     # warmup >= 2: the loop below holds the previous result while the next one is computed, so the pooled page-locked
     # output buffers ping-pong between two sets; both must exist before the clock starts (cudaHostAlloc of 2.5 GB ~ 1 s)
@@ -445,6 +491,8 @@ def run_ours(args, rank, world):
         I.set_gather("all")
         dev_chunks = 4
     dev = timed_device_steps(I, plumb, method, args.steps, warm, sampler, chunks=dev_chunks)
+    if args.dump_outputs and rank == 0:      # gather='all' above: rank 0 holds the whole result
+        dump_outputs(I, args.dump_outputs)
     value = n_points / (dev["ms_per_step"] * 1e-3)
     lo, hi = ctx.scalar("row_lo"), ctx.scalar("row_hi")
     compute_only, k4, gather_after = None, None, None
@@ -594,7 +642,13 @@ def main():
     ap.add_argument("--gather", default="host", choices=["host", "all"],
                     help="N > 1, e2e: where the row blocks meet (host: shared host mapping; all: every GPU, over NCCL)")
     ap.add_argument("--stream-chunks", type=int, default=8, help="node chunks of the e2e pipeline (0 = plain count + fetch)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="--impl ours: after the timed steps, write a seeded sample of the last step's result as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the result of this repository's arm (--impl ours)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.gpus != world:

@@ -8,6 +8,9 @@ Fixtures
   <name>.npz            synthetic mesh (points, one cell array per type, cell/point data) and every
                         output of the reference on it: Grid arrays, and for idw / ls / gls the CSR
                         (indptr, indices, data) and the neumann vector.
+  reference_digests.json, reference_gls_<mesh>.npz
+                        outputs of the reference on the meshes of the tests that compare with it, as digests
+                        and a sample of GLS rows (--digests; see make_digests).
   accuracy_hexa.json    the reference's own published known-answer numbers: relative L2 errors at interior
                         nodes on unit-cube n^3 hexahedral meshes, copied from
                         /root/reference/tests/results/yaml/accuracy.yaml (hexa rows; ALH :2-41, FAN :148-187,
@@ -145,5 +148,115 @@ def main():
                "table": table}, open(os.path.join(HERE, "accuracy_hexa.json"), "w"), indent=1)
 
 
+# ------------------------------------------------------------------------------------------------------------
+# Digests: the outputs of the reference on the meshes of the tests that compare with it on fresh meshes
+# (tests/test_oracle.py) and at size (tests/test_gpu_golden.py, tests/test_gpu_at_size.py), stored so that those
+# comparisons need nothing outside the repository.  Every array is stored as a digest (tests/helpers.py), which
+# settles a bit-exact comparison; GLS weights, compared within a tolerance, are stored as a seeded row sample.
+#
+#     python tests/golden/make_golden.py --digests [--source reference|oracle]
+#
+# --source oracle takes the outputs from the C oracle instead of the compiled reference; the source used is recorded.
+# On SMALL_CASES and EDGE_CASES the oracle's outputs were equal to the compiled reference's bit for bit (every Grid
+# array, every CSR of IDW / LS / GLS, the neumann vectors, the edge tables: test_oracle.py compared them directly), so
+# both sources write the same digests there.  AT_SIZE_CASES run the same C code and the same scipy DGELS on larger
+# meshes of the same generator.
+# ------------------------------------------------------------------------------------------------------------
+SMALL_CASES = [("tet", 6, {}), ("hex", 7, {}), ("mixed", 8, {"a": 2, "b": 4}), ("hex", 5, {"perturb": 0.2}),
+               ("tet", 1, {}), ("hex", 1, {}), ("quad2d", 6, {}), ("tri2d", 6, {"perturb": 0.2}),
+               ("tet", 6, {"scramble": True}), ("mixed", 8, {"a": 2, "b": 4, "scramble": True})]
+EDGE_CASES = [("tet", 5, {}), ("mixed", 8, {"a": 2, "b": 4}), ("tri2d", 7, {})]
+AT_SIZE_CASES = [("tet", 40, {}), ("tet", 69, {}), ("hex", 128, {})]
+GLS_SAMPLE = (100, 280, 20)        # Neumann boundary / interior / Dirichlet nodes of the stored GLS rows
+DIGESTS = os.path.join(HERE, "reference_digests.json")
+
+
+def case_key(kind, n, kw):
+    return "-".join([kind, str(n)] + [f"{k}={kw[k]}" for k in sorted(kw)])
+
+
+def gls_sample_path(key):
+    return os.path.join(HERE, f"reference_gls_{key}.npz")
+
+
+def mesh_digest(mesh):
+    sys.path.insert(0, os.path.dirname(HERE))
+    from helpers import digest
+    parts = [digest(mesh.points)] + [c.type + digest(c.data) for c in mesh.cells]
+    parts += [k + digest(np.concatenate([np.ravel(v) for v in mesh.cell_data[k]])) for k in sorted(mesh.cell_data)]
+    parts += [k + digest(mesh.point_data[k]) for k in sorted(mesh.point_data)]
+    return digest(np.frombuffer(" ".join(parts).encode(), dtype=np.uint8))
+
+
+def gls_sample_nodes(boundary_points, flags, rng):
+    bp = np.asarray(boundary_points) != 0
+    processed = ~(bp & (flags == 0))
+    groups = (np.nonzero(processed & bp)[0], np.nonzero(~bp)[0], np.nonzero(~processed)[0])
+    return np.sort(np.concatenate([rng.choice(g, size=min(len(g), k), replace=False) for g, k in zip(groups, GLS_SAMPLE)]))
+
+
+def outputs_digests(I, grid_arrays=GRID_ARRAYS):
+    from helpers import digest
+    g = I.grid
+    out = {"grid_scalars": {s: int(getattr(g, s)) for s in GRID_SCALARS},
+           "grid": {a: digest(getattr(g, a)) for a in grid_arrays}}
+    results = {}
+    for method in ("idw", "ls", "gls"):
+        W, nv = I.interpolate("u", method)
+        results[method] = (W, np.asarray(nv))
+        out[method] = {"indptr": digest(W.indptr), "indices": digest(W.indices), "nan": digest(np.isnan(W.data))}
+        if method != "gls":
+            out[method].update(data=digest(W.data), neumann=digest(nv))
+    return out, results
+
+
+def make_digests(source):
+    sys.path.insert(0, os.path.dirname(HERE))
+    if source == "reference" and oracle.load_reference() is None:
+        sys.exit("compiled reference not available: run `python oracle/build_ref.py` first, or pass --source oracle")
+
+    def interpolator(mesh, build_edges=False):
+        if source == "reference":
+            ninpol = oracle.load_reference()
+            I = ninpol.Interpolator(build_edges=True) if build_edges else ninpol.Interpolator()
+            I.load_mesh(mesh_obj=oracle.to_reference_mesh(mesh))
+            return I
+        return oracle.OracleInterpolator().load_mesh(mesh, build_edges=build_edges)
+
+    from helpers import digest
+    doc = {"source": "compiled reference (oracle/_ref)" if source == "reference" else
+           "C oracle (oracle/), equal to the compiled reference bit for bit on these meshes",
+           "small": {}, "edges": {}, "at_size": {}}
+    for kind, n, kw in SMALL_CASES:
+        mesh = meshgen.make_case(kind, n, **kw)
+        d, res = outputs_digests(interpolator(mesh))
+        W, nv = res["gls"]
+        d["gls"].update(data=digest(W.data), neumann=digest(nv))     # the oracle's GLS is the reference's bit for bit
+        doc["small"][case_key(kind, n, kw)] = dict(mesh=mesh_digest(mesh), **d)
+    for kind, n, kw in EDGE_CASES:
+        mesh = meshgen.make_case(kind, n, **kw)
+        g = interpolator(mesh, build_edges=True).grid
+        doc["edges"][case_key(kind, n, kw)] = {"mesh": mesh_digest(mesh), "n_edges": int(g.n_edges),
+                                               "inedel": digest(g.inedel), "inpoed": digest(g.inpoed)}
+    for kind, n, kw in AT_SIZE_CASES:
+        key = case_key(kind, n, kw)
+        mesh = meshgen.make_case(kind, n, **kw)
+        I = interpolator(mesh)
+        d, res = outputs_digests(I)
+        doc["at_size"][key] = dict(mesh=mesh_digest(mesh), **d)
+        W, nv = res["gls"]
+        flags = np.asarray(mesh.point_data["neumann_flag_u"]).astype(np.int64)
+        nodes = gls_sample_nodes(I.grid.boundary_points, flags, np.random.default_rng(20261020))
+        take = np.concatenate([np.arange(W.indptr[p], W.indptr[p + 1]) for p in nodes])
+        np.savez_compressed(gls_sample_path(key), nodes=nodes.astype(np.int64), row_nnz=np.diff(W.indptr)[nodes].astype(np.int64),
+                            indices=W.indices[take].astype(np.int64), data=W.data[take], neumann=nv[nodes])
+        print(key, "nodes", I.grid.n_points, "gls sample", len(nodes), os.path.getsize(gls_sample_path(key)), "bytes", flush=True)
+    with open(DIGESTS, "w") as f:
+        json.dump(doc, f, indent=1, sort_keys=True)
+
+
 if __name__ == "__main__":
-    main()
+    if "--digests" in sys.argv:
+        make_digests(sys.argv[sys.argv.index("--source") + 1] if "--source" in sys.argv else "reference")
+    else:
+        main()

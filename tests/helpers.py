@@ -16,6 +16,22 @@ GOLDEN_CASES = ("tet_n4", "hex_n4", "hex_n3_perturbed", "mixed_n6")
 GLS_TOL = 1e-12   # BASELINE.json north_star: <= 1e-12 relative weight error in FP64
 
 
+def digest(a):
+    """sha256 of an array's shape and values in a canonical form (integers as int64, floats as float64 with -0.0 as +0.0
+    and one NaN): two arrays have equal digests exactly when they have the same shape and np.array_equal(a, b,
+    equal_nan=True) holds."""
+    import hashlib
+    a = np.asarray(a)
+    if a.dtype.kind == "f":
+        a = a.astype(np.float64) + 0.0
+        a = np.where(np.isnan(a), np.nan, a)
+    else:
+        a = a.astype(np.int64)
+    h = hashlib.sha256(str(a.shape).encode())
+    h.update(np.ascontiguousarray(a).tobytes())
+    return h.hexdigest()
+
+
 def load_golden(name):
     sys.path.insert(0, GOLDEN)
     import make_golden
@@ -55,3 +71,41 @@ def check_against_golden(I, d, gls_tol=GLS_TOL, exact_gls=False):
         else:
             assert np.array_equal(W.data, d[method + "_data"], equal_nan=True), method
             assert np.array_equal(np.asarray(nv), d[method + "_neumann"]), method
+
+
+def load_reference_outputs(kind, n, kw):
+    """(mesh, digests, GLS row sample) of the reference's outputs on meshgen.make_case(kind, n, **kw), as stored by
+    tests/golden/make_golden.py --digests."""
+    import json
+    sys.path.insert(0, GOLDEN)
+    import make_golden
+    from ninpol_b200 import meshgen
+    key = make_golden.case_key(kind, n, kw)
+    with open(make_golden.DIGESTS) as f:
+        d = json.load(f)["at_size"][key]
+    mesh = meshgen.make_case(kind, n, **kw)
+    assert make_golden.mesh_digest(mesh) == d["mesh"], "the mesh generator no longer makes the stored mesh"
+    return mesh, d, dict(np.load(make_golden.gls_sample_path(key)))
+
+
+def check_against_reference_outputs(I, d, sample):
+    """Every Grid array, the IDW / LS CSR and neumann vectors and the GLS structure bit for bit against the stored
+    digests.  Returns the GLS result and, for the stored sample of rows, (row pointer, CUDA values)."""
+    g = I.grid
+    for s in GRID_SCALARS:
+        assert getattr(g, s) == d["grid_scalars"][s], s
+    for a in GRID_ARRAYS:
+        assert digest(getattr(g, a)) == d["grid"][a], a
+    for method in ("idw", "ls", "gls"):
+        W, nv = I.interpolate("u", method)
+        want = d[method]
+        assert digest(W.indptr) == want["indptr"] and digest(W.indices) == want["indices"], method
+        assert digest(np.isnan(W.data)) == want["nan"], method
+        if method != "gls":
+            assert digest(W.data) == want["data"] and digest(nv) == want["neumann"], method
+    nodes = sample["nodes"]
+    ptr = np.concatenate([[0], np.cumsum(sample["row_nnz"])])
+    assert np.array_equal(np.diff(W.indptr)[nodes], sample["row_nnz"])
+    take = np.concatenate([np.arange(W.indptr[p], W.indptr[p + 1]) for p in nodes])
+    assert np.array_equal(W.indices[take], sample["indices"])
+    return W, np.asarray(nv), ptr, W.data[take]

@@ -1,9 +1,10 @@
-"""CUDA path against the committed golden fixtures (outputs of the compiled reference) and, when
-oracle/_ref travelled to the box, against the compiled reference itself on a larger mesh."""
-import numpy as np
+"""CUDA path against the committed golden fixtures (outputs of the compiled reference), and against the reference's
+outputs on a larger mesh stored as digests and a row sample."""
+import types
+
 import pytest
 
-from helpers import GLS_TOL, GOLDEN_CASES, GRID_ARRAYS, check_against_golden, load_golden, row_normwise_error
+from helpers import GLS_TOL, GOLDEN_CASES, check_against_golden, load_golden, row_normwise_error
 
 pytestmark = pytest.mark.gpu
 
@@ -40,25 +41,12 @@ def test_cuda_reproduces_published_accuracy():
 
 
 def test_cuda_matches_compiled_reference_when_available():
-    import oracle
-    ref = oracle.load_reference()
-    if ref is None:
-        pytest.skip("oracle/_ref not present on this box")
+    """Kuhn tets n = 40 (384,000 cells / 68,921 nodes, 50 % Neumann hull nodes) against the compiled reference's outputs
+    stored under tests/golden/: everything bit for bit but the GLS weights, which a seeded sample of rows bounds."""
     import ninpol_b200
-    from ninpol_b200 import meshgen
-    mesh = meshgen.make_case("tet", 40)       # 384,000 cells / 68,921 nodes, 50 % Neumann hull nodes
-    R = ref.Interpolator()
-    R.load_mesh(mesh_obj=oracle.to_reference_mesh(mesh))
+    from helpers import check_against_reference_outputs, load_reference_outputs
+    mesh, d, sample = load_reference_outputs("tet", 40, {})
     I = ninpol_b200.Interpolator()
     I.load_mesh(mesh_obj=mesh)
-    for a in GRID_ARRAYS:
-        assert np.array_equal(np.asarray(getattr(I.grid, a)), np.asarray(getattr(R.grid, a))), a
-    for method in ("idw", "ls", "gls"):
-        W, nv = I.interpolate("u", method)
-        Wr, nvr = R.interpolate("u", method)
-        assert np.array_equal(W.indptr, Wr.indptr) and np.array_equal(W.indices, Wr.indices)
-        if method == "gls":
-            assert row_normwise_error(W, W.indptr, Wr.data) <= GLS_TOL
-        else:
-            assert np.array_equal(W.data, Wr.data, equal_nan=True)
-            assert np.array_equal(nv, np.asarray(nvr))
+    W, nv, ptr, got = check_against_reference_outputs(I, d, sample)
+    assert row_normwise_error(types.SimpleNamespace(data=got), ptr, sample["data"]) <= GLS_TOL

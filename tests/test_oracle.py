@@ -1,6 +1,6 @@
 """CPU tests of the oracle (test infrastructure): it must agree with the reference's golden vectors,
-with the fixtures generated from the compiled reference, and — where oracle/_ref is present — with the
-compiled reference itself on fresh meshes."""
+with the fixtures generated from the compiled reference, and with the reference's outputs on further meshes
+(2-D, single-cell, renumbered, edge tables), stored as digests."""
 import json
 import os
 import sys
@@ -8,7 +8,7 @@ import sys
 import numpy as np
 import pytest
 
-from helpers import GOLDEN, GOLDEN_CASES, GRID_ARRAYS, GRID_SCALARS, check_against_golden, load_golden
+from helpers import GOLDEN, GOLDEN_CASES, GRID_ARRAYS, GRID_SCALARS, check_against_golden, digest, load_golden
 
 import oracle
 from ninpol_b200 import meshgen
@@ -48,28 +48,29 @@ def test_oracle_linear_exactness():
         assert make_golden.interior_l2(W, mesh, sol, "LIN", O.grid.boundary_points) < 1e-14
 
 
-REF = oracle.load_reference()
-
-
-@pytest.mark.skipif(REF is None, reason="compiled reference (oracle/_ref) not built in this checkout")
-@pytest.mark.parametrize("kind,n,kw", [("tet", 6, {}), ("hex", 7, {}), ("mixed", 8, {"a": 2, "b": 4}), ("hex", 5, {"perturb": 0.2}),
-                                       ("tet", 1, {}), ("hex", 1, {}), ("quad2d", 6, {}), ("tri2d", 6, {"perturb": 0.2}),
-                                       ("tet", 6, {"scramble": True}), ("mixed", 8, {"a": 2, "b": 4, "scramble": True})])
-def test_oracle_matches_compiled_reference(kind, n, kw):
+def _stored(section, kind, n, kw):
+    with open(make_golden.DIGESTS) as f:
+        doc = json.load(f)[section]
+    d = doc[make_golden.case_key(kind, n, kw)]
     mesh = meshgen.make_case(kind, n, **kw)
-    I = REF.Interpolator()
-    I.load_mesh(mesh_obj=oracle.to_reference_mesh(mesh))
+    assert make_golden.mesh_digest(mesh) == d["mesh"], "the mesh generator no longer makes the stored mesh"
+    return mesh, d
+
+
+@pytest.mark.parametrize("kind,n,kw", make_golden.SMALL_CASES)
+def test_oracle_matches_compiled_reference(kind, n, kw):
+    """Every output of the oracle equals the compiled reference's (stored as digests, tests/golden/make_golden.py)."""
+    mesh, d = _stored("small", kind, n, kw)
     O = oracle.OracleInterpolator().load_mesh(mesh)
     for s in GRID_SCALARS:
-        assert getattr(I.grid, s) == getattr(O.grid, s), s
+        assert getattr(O.grid, s) == d["grid_scalars"][s], s
     for a in GRID_ARRAYS:
-        assert np.array_equal(np.asarray(getattr(I.grid, a)), getattr(O.grid, a)), a
+        assert digest(getattr(O.grid, a)) == d["grid"][a], a
     for method in ("idw", "ls", "gls"):
-        W, nv = I.interpolate("u", method)
-        Wo, nvo = O.interpolate("u", method)
-        assert np.array_equal(W.indptr, Wo.indptr) and np.array_equal(W.indices, Wo.indices)
-        assert np.array_equal(W.data, Wo.data, equal_nan=True), method
-        assert np.array_equal(np.asarray(nv), nvo)
+        W, nv = O.interpolate("u", method)
+        want = d[method]
+        for name, got in (("indptr", W.indptr), ("indices", W.indices), ("data", W.data), ("neumann", nv)):
+            assert digest(got) == want[name], (method, name)
 
 
 def test_release_build_diffusion_magnitude():
@@ -80,13 +81,10 @@ def test_release_build_diffusion_magnitude():
     assert np.array_equal(dm, (1 - 3 / tr) ** 2)
 
 
-@pytest.mark.skipif(REF is None, reason="compiled reference (oracle/_ref) not built in this checkout")
-@pytest.mark.parametrize("kind,n,kw", [("tet", 5, {}), ("mixed", 8, {"a": 2, "b": 4}), ("tri2d", 7, {})])
+@pytest.mark.parametrize("kind,n,kw", make_golden.EDGE_CASES)
 def test_oracle_edges_match_compiled_reference(kind, n, kw):
-    mesh = meshgen.make_case(kind, n, **kw)
-    I = REF.Interpolator(build_edges=True)
-    I.load_mesh(mesh_obj=oracle.to_reference_mesh(mesh))
+    mesh, d = _stored("edges", kind, n, kw)
     O = oracle.OracleInterpolator().load_mesh(mesh, build_edges=True)
-    assert I.grid.n_edges == O.grid.n_edges
-    assert np.array_equal(np.asarray(I.grid.inedel), O.grid.inedel)
-    assert np.array_equal(np.asarray(I.grid.inpoed), O.grid.inpoed)
+    assert O.grid.n_edges == d["n_edges"]
+    assert digest(O.grid.inedel) == d["inedel"]
+    assert digest(O.grid.inpoed) == d["inpoed"]
