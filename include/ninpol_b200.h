@@ -142,6 +142,20 @@ int npb_set_point_flags_f64_range(npb_ctx *ctx, const double *flag_slice, int64_
 int npb_interpolate_count(npb_ctx *ctx, int method, int64_t *nnz);
 int npb_interpolate_fetch(npb_ctx *ctx, int32_t *indptr, int32_t *indices, double *data, double *neumann);
 
+/* K5 — nodal values from the resident weights (no reference counterpart; the reference's callers multiply the CSR
+ * by the cell field with scipy, `W @ u`).
+ * out[p, c] = sum over the entries j of row p in ascending order of data[j] * values[indices[j], c], for c < n_cols,
+ * using the CSR of `method` that the last npb_interpolate_count / npb_interpolate_run left on the device.  Each sum
+ * starts at +0.0 and every product and addition is rounded on its own: bit-identical to scipy's csr_matvec(s).
+ * values [n_elems, n_cols] and out [n_points, n_cols]: float64, row-major, host memory (pageable or page-locked).
+ * NPB_ERR_STATE when no CSR of `method` is resident (c->counted false or c->method != method): every change of the
+ * inputs (flags, cell fields, partition, gather mode, mesh, npb_interpolate_dense) voids it.  When world > 1 this is
+ * collective: each rank reads only the rows of `values` its nodes refer to (npb_partition_elem_range), computes its
+ * own rows, and the row blocks of the result are all-gathered, so every rank's `out` holds all n_points rows in every
+ * gather mode; no CSR block moves between the GPUs or to the host.  Timings: "h2d_apply" "apply" "apply_gather"
+ * "d2h_apply" (and "k3_fill" when the rows still had to be written). */
+int npb_apply(npb_ctx *ctx, int method, const double *values, int64_t n_cols, double *out);
+
 /* The plug-in's own output, for callers that sit where Interpolator.prepare_interpolator sits
  * (interpolator.pyx:631-670): dense weights [n_points, MX_ELEMENTS_PER_POINT] (row stride
  * MX_ELEMENTS_PER_POINT, column k of row p <-> esup[esup_ptr[p] + k], untouched entries 0) and neumann_ws

@@ -43,6 +43,7 @@ _SIGNATURES = {
     "npb_interpolate_run": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int, ctypes.c_int] + [ctypes.c_void_p] * 6
                             + [ctypes.c_int64, _c_i64p, ctypes.POINTER(ctypes.c_int)]),
     "npb_interpolate_streamed": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int, ctypes.c_int] + [ctypes.c_void_p] * 6 + [ctypes.c_int64, _c_i64p]),
+    "npb_apply": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_int64, ctypes.c_void_p]),
     "npb_timing": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_char_p, ctypes.POINTER(ctypes.c_double)]),
     "npb_launch_count": (ctypes.c_int, [ctypes.c_void_p, _c_i64p]),
     "npb_check_guards": (ctypes.c_int, [ctypes.c_void_p, _c_i64p, _c_i64p]),
@@ -236,6 +237,15 @@ class Context:
 
     def interpolate_fetch(self, indptr, indices, data, neumann):
         check(self.lib.npb_interpolate_fetch(self.handle, _ptr(indptr), _ptr(indices), _ptr(data), _ptr(neumann)))
+
+    def apply(self, method, values, out):
+        """out[:] = W @ values with the CSR of `method` resident on the device (npb_apply).  values [n_elems, k] and
+        out [n_points, k]: float64, C-contiguous (1-D: k = 1).  Collective when world > 1."""
+        assert values.dtype == np.float64 and out.dtype == np.float64
+        assert values.flags.c_contiguous and out.flags.c_contiguous
+        k = 1 if values.ndim == 1 else int(values.shape[1])
+        assert values.ndim in (1, 2) and out.ndim == values.ndim and out.shape[1:] == values.shape[1:]
+        check(self.lib.npb_apply(self.handle, METHOD_IDS[method], _ptr(values), k, _ptr(out)))
 
     # --- measurement ---
     def timing(self, name):

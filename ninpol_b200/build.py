@@ -33,6 +33,7 @@ UNITS = {
     "k3_emit.cu": [],
     "k4_shard.cu": [],
     "pipeline.cu": [],
+    "k5_apply.cu": ["-fmad=false"],
 }
 
 

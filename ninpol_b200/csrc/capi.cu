@@ -298,6 +298,7 @@ static void free_mesh(npb_ctx *c)
     c->chunk_efirst.clear();
     c->chunk_elast.clear();
     c->plan_failed[0] = c->plan_failed[1] = c->plan_failed[2] = false;
+    c->apply_range_ok = false;
 }
 
 extern "C" int npb_create(int device, npb_ctx **out)
@@ -363,6 +364,8 @@ extern "C" int npb_destroy(npb_ctx *c)
     if (c->scan_tmp) { npb_guard_forget(c->scan_tmp); cudaFree(c->scan_tmp); }
     if (c->part_tmp) { npb_guard_forget(c->part_tmp); cudaFree(c->part_tmp); }
     if (c->gls_ws) { npb_guard_forget(c->gls_ws); cudaFree(c->gls_ws); }
+    if (c->apply_x) { npb_guard_forget(c->apply_x); cudaFree(c->apply_x); }
+    if (c->apply_y) { npb_guard_forget(c->apply_y); cudaFree(c->apply_y); }
     if (c->counters) cudaFree(c->counters);
     if (c->h_small) cudaFreeHost(c->h_small);
     for (int i = 0; i < 2; i++) {
@@ -407,6 +410,7 @@ static int refresh_range(npb_ctx *c)
     c->wlen = (i64)b[1] - b[0];
     c->counted = false;
     c->plan_chunks = 0;   // chunk boundaries follow the rank bounds
+    c->apply_range_ok = false;
     return NPB_OK;
 }
 
@@ -1026,6 +1030,66 @@ extern "C" int npb_interpolate_fetch(npb_ctx *c, int32_t *indptr, int32_t *indic
         tm.stop();
     }
     NPB_CUDA(cudaStreamSynchronize(s));
+    return NPB_OK;
+}
+
+// ------------------------------------------------------------------------------------------------
+// K5 — nodal values W @ values from the CSR left on the device by the last count / run
+// ------------------------------------------------------------------------------------------------
+extern "C" int npb_apply(npb_ctx *c, int method, const double *values, int64_t n_cols, double *out)
+{
+    if (!c || n_cols < 0 || (n_cols > 0 && (!values || !out))) return NPB_ERR_ARG;
+    if (!c->counted || c->method != method) {
+        npb_set_error("npb_apply: no weights of method %d are resident (run npb_interpolate_count or npb_interpolate_run "
+                      "for the current inputs first)", method);
+        return NPB_ERR_STATE;
+    }
+    if (n_cols == 0) return NPB_OK;
+    NPB_CUDA(cudaSetDevice(c->device));
+    if (!c->filled) {   // the two-pass count (exact-zero fallback, or world > 1) left the rows unwritten
+        NPB_TRY(npb_ensure_out(c, (size_t)c->nnz));
+        NpbTimer tm(c, "k3_fill");
+        NPB_TRY(npb_k3_fill(c, c->lo, c->hi));
+        tm.stop_lazy();
+        c->filled = true;
+    }
+    // this rank's nodes read the values of the elements in their esup rows only: upload that slice
+    i64 first = 0, last = c->n_elems - 1;
+    if (c->world > 1) {
+        if (!c->apply_range_ok) {
+            int64_t f = 0, l = -1;
+            NPB_TRY(npb_partition_elem_range(c, &f, &l));
+            c->apply_first = f;
+            c->apply_last = l;
+            c->apply_range_ok = true;
+        }
+        first = c->apply_first;
+        last = c->apply_last;
+    }
+    const i64 n_up = last >= first ? last - first + 1 : 0;
+    NPB_TRY(npb_ensure((void **)&c->apply_x, &c->apply_x_cap, sizeof(double) * (size_t)(c->n_elems * n_cols)));
+    NPB_TRY(npb_ensure((void **)&c->apply_y, &c->apply_y_cap, sizeof(double) * (size_t)(c->n_points * n_cols)));
+    {
+        NpbTimer tm(c, "h2d_apply");
+        NPB_TRY(npb_h2d(c, c->apply_x + first * n_cols, values + first * n_cols, sizeof(double) * (size_t)(n_up * n_cols)));
+        tm.stop_lazy();
+    }
+    {
+        NpbTimer tm(c, "apply");
+        NPB_TRY(npb_k5_apply(c, c->lo, c->hi, c->apply_x, n_cols, c->apply_y));
+        tm.stop_lazy();
+    }
+    if (c->world > 1) {
+        NpbTimer tm(c, "apply_gather");
+        NPB_TRY(npb_k4_gather_rows(c, c->apply_y, n_cols));
+        tm.stop_lazy();
+    }
+    {
+        NpbTimer tm(c, "d2h_apply");
+        NPB_TRY(npb_d2h(c, out, c->apply_y, sizeof(double) * (size_t)(c->n_points * n_cols)));
+        tm.stop();
+    }
+    NPB_CUDA(cudaStreamSynchronize(c->stream));
     return NPB_OK;
 }
 

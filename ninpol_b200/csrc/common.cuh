@@ -148,6 +148,11 @@ struct npb_ctx {
     std::vector<i64> chunk_node, chunk_nz;   // [world * K + 1] node / nnz boundaries of every rank's chunks
     std::vector<i64> chunk_efirst, chunk_elast;   // [K] element range this rank's chunk k reads (empty: not computed yet)
     bool gathered = false;               // indices / data / neumann of ALL ranks are on this device (gather = all)
+    // npb_apply (k5_apply.cu): the values uploaded for this rank's rows and the result rows, [.., n_cols] row-major
+    double *apply_x = nullptr, *apply_y = nullptr;
+    size_t apply_x_cap = 0, apply_y_cap = 0;
+    bool apply_range_ok = false;         // apply_first / apply_last hold npb_partition_elem_range for the current partition
+    i64 apply_first = 0, apply_last = -1;
 };
 
 // ---- helpers implemented in capi.cu ----
@@ -194,6 +199,8 @@ __global__ void k_copy_int(int *dst, const int *src);    // capi.cu   // device 
 int npb_minmax_i32(npb_ctx *c, const int32_t *in, i64 n, int32_t *h_min, int32_t *h_max);
 int npb_k4_gather_counts(npb_ctx *c);
 int npb_k4_gather_blocks(npb_ctx *c);
+int npb_k4_gather_rows(npb_ctx *c, double *rows, i64 n_cols);
+int npb_k5_apply(npb_ctx *c, i64 lo, i64 hi, const double *x, int64_t k, double *out);
 int npb_export_array(npb_ctx *c, const char *name, void *out, i64 cap);
 // cudaMalloc'ed temporary that is freed when it goes out of scope (error returns included)
 struct NpbTmp {

@@ -198,6 +198,26 @@ int npb_k4_gather_blocks(npb_ctx *c)
     return NPB_OK;
 }
 
+// all-gather of the row blocks of a [n_points, n_cols] float64 array (npb_apply's result): rank r owns the rows
+// [bounds[r], bounds[r + 1]).  One group of ncclSend / ncclRecv, as in npb_k4_gather_blocks, whatever the gather mode:
+// the result is n_points * n_cols doubles, small next to the CSR.
+int npb_k4_gather_rows(npb_ctx *c, double *rows, i64 n_cols)
+{
+    if (c->world == 1) return NPB_OK;
+    NcclApi *api = c->nccl;
+    ncclComm_t comm = (ncclComm_t)c->comm;
+    const i64 mb = c->bounds[c->rank] * n_cols, mn = (c->bounds[c->rank + 1] - c->bounds[c->rank]) * n_cols;
+    NPB_NCCL(api->GroupStart());
+    for (int r = 0; r < c->world; r++) {
+        if (r == c->rank) continue;
+        const i64 b = c->bounds[r] * n_cols, n = (c->bounds[r + 1] - c->bounds[r]) * n_cols;
+        if (mn > 0) NPB_NCCL(api->Send(rows + mb, (size_t)mn, ncclFloat64, r, comm, c->stream));
+        if (n > 0) NPB_NCCL(api->Recv(rows + b, (size_t)n, ncclFloat64, r, comm, c->stream));
+    }
+    NPB_NCCL(api->GroupEnd());
+    return NPB_OK;
+}
+
 // Every rank contributes one int; *any = 1 when some rank's is non-zero: ONE 4-byte ncclAllReduce (sum) on the
 // compute stream - the only exchange of a planned IDW / LS step - whose result comes back through the mapped block.
 __global__ void k_fold_flags(int *dst, const int *bad2, int host_flag) { *dst = (bad2[0] != 0 || bad2[1] != 0 || host_flag != 0) ? 1 : 0; }

@@ -6,6 +6,7 @@ Same constructor keywords, methods and attributes as the reference class
     I = Interpolator(name="interpolator", logging=False, build_edges=False)
     I.load_mesh(mesh_obj=mesh)                       # or filename=... when meshio is installed
     W, neumann = I.interpolate("pressure", "gls")    # scipy CSR (n_nodes, n_elements), ndarray (n_nodes,)
+    u_nodes = I.nodal_values("pressure", "gls")     # W @ u on the GPU, bit for bit; the weights stay resident
     I.supported_methods                              # {"gls": ..., "idw": ..., "ls": ...}
 
 The host side only ingests the mesh object (vectorised numpy instead of the reference's per-item Python
@@ -63,6 +64,7 @@ class _Method:
         nw = np.asarray(neumann_ws)
         if w.shape != (n, mx) or nw.shape != (n,) or w.dtype != DTYPE_F or nw.dtype != DTYPE_F:
             raise ValueError(f"weights must be float64 [{n}, {mx}] and neumann_ws float64 [{n}] (interpolator.pyx:645-651)")
+        I._weights_key = None              # the dense path below voids the resident CSR
         I._stage_inputs(self.method, variable, variable_to_index, cells_data, points_data)
         # the kernels' esup-indexed values go straight into the caller's dense rows (npb_interpolate_dense):
         # nothing is rebuilt from the zero-eliminated CSR
@@ -178,6 +180,8 @@ class Interpolator:
         self._partition_key = None
         self._flag_mask, self._flag_version, self._elem_range_key, self._elem_range = None, 0, None, (0, -1)
         self._shared, self._shared_reg, self._mesh_serial = None, None, 0
+        # (method, variable, _data_version, _mesh_serial) of the CSR resident on the device, for nodal_values
+        self._weights_key = None
         self.last_timings = {}
 
     def _dense_view(self, kind):
@@ -315,6 +319,7 @@ class Interpolator:
         self._partition_key = None
         self._shared, self._shared_reg = None, None      # gather="host": a new mapping per mesh
         self._mesh_serial += 1
+        self._weights_key = None
         self.logger.log(f"Mesh loaded successfully: {n_points} points and {n_elems} elements.")
         if not cached and filename != "":
             little_hash = hex(os.path.getsize(filename))
@@ -598,6 +603,7 @@ class Interpolator:
         if gather not in ("all", "root", "host"):
             raise ValueError("gather must be 'all', 'root' or 'host'")
         self.gather = gather
+        self._weights_key = None           # npb_set_gather voids the resident CSR
         if self.comm.world > 1:
             self._ctx.set_gather(gather)
 
@@ -630,8 +636,10 @@ class Interpolator:
 
     def invalidate_inputs(self):
         """Forget which per-variable inputs are resident on the device: the next interpolate() uploads
-        the flags (and, for GLS, permeability + diff_mag) again from host memory."""
+        the flags (and, for GLS, permeability + diff_mag) again from host memory, and nodal_values() recomputes the
+        weights."""
         self._staged = None
+        self._weights_key = None
 
     def _set_partition(self, method):
         if self.comm.world == 1:
@@ -652,14 +660,26 @@ class Interpolator:
             return np.empty(n, dtype=dtype)
         return self._pool.take(name, n, dtype)
 
-    def _run_pipeline(self, method, fields):
+    def _run_pipeline(self, method, fields, fetch=True):
         """npb_interpolate_run: plan, then chunks of this rank's nodes through upload / compute / gather / download
         streams.  Returns None when the plan was voided (an exact-zero weight somewhere): the caller falls back to the
-        two-pass path - every rank takes the same decision."""
+        two-pass path - every rank takes the same decision.  fetch=False: the CSR stays on the device (one GPU);
+        returns its nnz."""
         g, ctx = self.grid, self._ctx
         n_points, cap = g.n_points, max(1, ctx.scalar("len_esup"))
         perm, dm = fields if fields is not None else (None, None)
         world = self.comm.world
+        # every rank must cut the same number of chunks (the NCCL gather is chunked alike): the rule uses global sizes
+        rule = min(self.min_chunk_nodes, self.min_chunk_nodes_gls) if method == "gls" else self.min_chunk_nodes
+        chunks = max(1, min(self.stream_chunks, n_points // (max(1, rule) * world)))
+        if not fetch:
+            nnz, fell_back = ctx.interpolate_run(method, chunks, perm, dm)
+            if fell_back:
+                return None
+            if perm is not None:
+                self.last_timings["h2d_input_bytes"] += perm.nbytes + dm.nbytes
+            self.last_timings.update({"streamed_ms": ctx.timing_or("streamed"), "nnz": nnz})
+            return nnz
         if world > 1 and self.gather == "host":
             so = self._shared_outputs()
             ctx.comm_barrier()        # every rank is done with the arrays of the previous call
@@ -669,9 +689,6 @@ class Interpolator:
             arrays = (self._out("indptr", n_points + 1, np.int32), self._out("indices", cap, np.int32),
                       self._out("data", cap, np.float64), self._out("neumann", n_points, np.float64))
             pinned = self.pinned_outputs
-        # every rank must cut the same number of chunks (the NCCL gather is chunked alike): the rule uses global sizes
-        rule = min(self.min_chunk_nodes, self.min_chunk_nodes_gls) if method == "gls" else self.min_chunk_nodes
-        chunks = max(1, min(self.stream_chunks, n_points // (max(1, rule) * world)))
         if pinned:
             nnz, fell_back = ctx.interpolate_run(method, chunks, perm, dm, *arrays)
         else:                         # pageable outputs: device-resident run, then the staged copies of fetch
@@ -699,9 +716,16 @@ class Interpolator:
         self.last_timings.update({"streamed_ms": ctx.timing_or("streamed"), "nnz": nnz})
         return out
 
-    def _run(self, method):
+    def _run(self, method, fetch=True):
         g = self.grid
         self._set_partition(method)
+        if not fetch:
+            # the two-pass count only: the rows stay on the device (world > 1: the ranks exchange row counts and
+            # neumann entries, no CSR block); npb_apply writes them if the count left them unwritten
+            nnz = self._ctx.interpolate_count(method)
+            t = self._ctx.timing_or
+            self.last_timings.update({"k2_ms": t("k2"), "k3_count_ms": t("k3_count"), "nnz": nnz})
+            return nnz
         if self.comm.world > 1 and self.gather == "host":
             so = self._shared_outputs()
             self._ctx.comm_barrier()        # every rank is done with the arrays of the previous call
@@ -730,33 +754,88 @@ class Interpolator:
         return indptr, indices, data, neumann
 
     def interpolate(self, variable, method, target_points=np.array([], dtype=DTYPE_I)):
-        if not self.is_grid_initialized:
-            raise ValueError("Grid not initialized. Please load a mesh first.")
-        if method not in self.supported_methods:
-            raise ValueError(f"Method '{method}' not supported. Supported methods are: {list(self.supported_methods.keys())}")
-        if variable not in self.variable_to_index["cells"]:
-            raise ValueError(f"Variable '{variable}' not found in cells data. Point -> Cell interpolation not supported yet.")
+        self._check_call(variable, method)
         data_index = self.variable_to_index["cells"][variable]
         if self.cells_data_dimensions[data_index] > 1:
             raise ValueError(f"Variable '{variable}' has more than one dimension. Vector data not supported yet.")
         self._check_targets(target_points)
         self.logger.log(f"Interpolating variable '{variable}' using method '{method}'")
-        piped = self.stream_chunks > 0 and not (self.comm.world > 1 and self.gather == "root")
-        fields = self._stage_inputs(method, variable, self.variable_to_index, self._rows["cells"], self._rows["points"],
-                                    defer_fields=piped and self.pin_inputs)
-        out = self._run_pipeline(method, fields) if piped else None
-        if out is None:
-            if fields is not None and not (self._ctx_has_fields()):
-                # the pipeline never ran (or gave up before its uploads): stage the cell fields the classic way
-                fields = None
-                self._stage_inputs(method, variable, self.variable_to_index, self._rows["cells"], self._rows["points"])
-            out = self._run(method)
-        if getattr(self, "_pending_key", None) is not None:
-            self._staged, self._pending_key = self._pending_key, None
-        indptr, indices, data, neumann = out
+        indptr, indices, data, neumann = self._compute_weights(variable, method, fetch=True)
         g = self.grid
         # the device emitted canonical CSR (sorted, zero-free, int32 index arrays): no conversion, no copy
         W = sp.csr_matrix((data, indices, indptr), shape=(g.n_points, g.n_elems), copy=False)
         W.has_sorted_indices = True
         W.has_canonical_format = True
         return W, neumann
+
+    def _check_call(self, variable, method):
+        """The argument checks interpolate() and nodal_values() share (interpolator.pyx:549-560)."""
+        if not self.is_grid_initialized:
+            raise ValueError("Grid not initialized. Please load a mesh first.")
+        if method not in self.supported_methods:
+            raise ValueError(f"Method '{method}' not supported. Supported methods are: {list(self.supported_methods.keys())}")
+        if variable not in self.variable_to_index["cells"]:
+            raise ValueError(f"Variable '{variable}' not found in cells data. Point -> Cell interpolation not supported yet.")
+
+    def _compute_weights(self, variable, method, fetch):
+        """Stages the inputs of (method, variable) and computes the CSR: the chunk pipeline where it applies, else (or when
+        an exact-zero weight voids its plan) the two-pass path.  fetch=True: returns the host arrays (indptr, indices, data,
+        neumann).  fetch=False: the CSR stays on the device for npb_apply, nothing is downloaded; with world > 1 only the
+        two-pass count runs, since the pipeline's gather = "all" would broadcast every block."""
+        self._weights_key = None
+        if fetch:
+            piped = self.stream_chunks > 0 and not (self.comm.world > 1 and self.gather == "root")
+        else:
+            piped = self.stream_chunks > 0 and self.comm.world == 1
+        fields = self._stage_inputs(method, variable, self.variable_to_index, self._rows["cells"], self._rows["points"],
+                                    defer_fields=piped and self.pin_inputs)
+        out = self._run_pipeline(method, fields, fetch) if piped else None
+        if out is None:
+            if fields is not None and not (self._ctx_has_fields()):
+                # the pipeline never ran (or gave up before its uploads): stage the cell fields the classic way
+                fields = None
+                self._stage_inputs(method, variable, self.variable_to_index, self._rows["cells"], self._rows["points"])
+            out = self._run(method, fetch)
+        if getattr(self, "_pending_key", None) is not None:
+            self._staged, self._pending_key = self._pending_key, None
+        self._weights_key = (method, variable, self._data_version, self._mesh_serial)
+        return out
+
+    def nodal_values(self, variable, method, values=None):
+        """Nodal values `W @ values`, where W is the CSR `interpolate(variable, method)` returns, computed on the GPU
+        from the resident weights: bit-identical to scipy's product (NaN included), without the CSR ever leaving the
+        device.  The weights stay resident between calls; a later call with the same (method, variable) and unchanged
+        inputs only uploads `values`, runs one kernel and downloads the result.
+
+        values: None (the cell data of `variable`: shape (n_elems,), or (n_elems, dim) for a vector variable, which
+        this method accepts), or any real array of shape (n_elems,) or (n_elems, k), converted to float64 like scipy
+        does.  Returns float64 of shape (n_points,) or (n_points, k).  With several GPUs every rank calls it and every
+        rank receives the full result, in every gather mode."""
+        self._check_call(variable, method)
+        g = self.grid
+        n_elems, n_points = g.n_elems, g.n_points
+        if values is None:
+            dim = int(self.cells_data_dimensions[self.variable_to_index["cells"][variable]])
+            row = np.asarray(self._rows["cells"][self.variable_to_index["cells"][variable]], dtype=DTYPE_F)
+            x = row[:n_elems * dim] if dim == 1 else row[:n_elems * dim].reshape(n_elems, dim)
+        else:
+            if np.iscomplexobj(values):
+                raise TypeError("nodal_values: complex values are not supported; pass the real and imaginary parts "
+                                "as separate columns")
+            x = np.asarray(values, dtype=DTYPE_F)
+            if x.ndim not in (1, 2) or x.shape[0] != n_elems:
+                raise ValueError(f"nodal_values: values must have shape ({n_elems},) or ({n_elems}, k), got {x.shape}")
+        x = np.ascontiguousarray(x)
+        if x.ndim == 2 and x.shape[1] == 0:
+            return np.empty((n_points, 0), dtype=DTYPE_F)
+        key = (method, variable, self._data_version, self._mesh_serial)
+        reused = self._weights_key == key
+        if not reused:
+            self._compute_weights(variable, method, fetch=False)
+        out = self._out("nodal", n_points * (1 if x.ndim == 1 else x.shape[1]), DTYPE_F)
+        out = out.reshape((n_points,) + x.shape[1:])
+        self._ctx.apply(method, x, out)
+        t = self._ctx.timing_or
+        self.last_timings.update({"nodal_h2d_ms": t("h2d_apply"), "nodal_apply_ms": t("apply"),
+                                  "nodal_d2h_ms": t("d2h_apply"), "nodal_weights_reused": reused})
+        return out
