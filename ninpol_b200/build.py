@@ -27,7 +27,6 @@ UNITS = {
     "k1_geometry.cu": ["-fmad=false"],
     "k2_idw_ls.cu": ["-fmad=false"],
     "k2_idw_ls_tile.cu": ["-fmad=false"],
-    "k2_tile_pipe.cu": ["-fmad=false"],
     "k2_gls.cu": [],
     "k2_gls_dense.cu": [],
     "k3_emit.cu": [],

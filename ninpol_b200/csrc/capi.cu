@@ -80,8 +80,8 @@ extern "C" int npb_check_guards(npb_ctx *c, int64_t *n_blocks, int64_t *n_damage
 int npb_alloc(npb_ctx *c, void **p, size_t bytes, bool owned_by_mesh)
 {
     *p = nullptr;
-    // 64 bytes of slack: TMA bulk copies of element-aligned slices are rounded out to 16-byte boundaries
-    // (k2_tile_pipe.cu) and may read up to 15 bytes past the last element
+    // 64 bytes of slack behind every block: guard mode arms its guard words there, and no kernel has been
+    // audited for reads past the end of its inputs
     NPB_CUDA(cudaMalloc(p, bytes + 64));
     if (owned_by_mesh) c->owned.push_back(*p);
     if (guards_on()) NPB_TRY(guard_arm(*p, bytes));

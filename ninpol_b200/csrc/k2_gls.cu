@@ -58,7 +58,7 @@ struct MfClass {
 #define MF_CLASS_TABLE {{0, 0, 0, 0}, {640, 8, 14, 3072}, {640, 12, 22, 6144}, {768, 16, 30, 8192}, {1664, 24, 40, 12288}, \
                         {1664, 32, 56, 18432}, {2560, 48, 80, 32768}, {4096, 64, 112, 49152}, {0, 0, 0, 0}}
 __constant__ MfClass c_mf[MF_NCLASS] = MF_CLASS_TABLE;
-static MfClass h_mf[MF_NCLASS] = MF_CLASS_TABLE;
+static const MfClass h_mf[MF_NCLASS] = MF_CLASS_TABLE;
 
 // group table entries: original groups (<= ecap + fcap_f), leaf contribution blocks and re-entered survivors of the
 // leaf phase (<= ecap together), one contribution block per general front (<= ecap)
@@ -1260,31 +1260,9 @@ int npb_k2_gls(npb_ctx *c, i64 lo, i64 hi)
     NPB_LAUNCH(c);
     k_gls_publish_sig<<<1, 32, 0, s>>>(sig, c->d_small + 44);
     NPB_LAUNCH(c);
-    {   // experiments: NPB_GLS_FCAP="class:doubles[,class:doubles...]" overrides the front sizes (re-read every pass)
-        static const MfClass defaults[MF_NCLASS] = MF_CLASS_TABLE;
-        MfClass want[MF_NCLASS];
-        memcpy(want, defaults, sizeof(want));
-        const char *fo = getenv("NPB_GLS_FCAP");
-        for (const char *q = fo; q && *q;) {
-            int k = atoi(q);
-            const char *col = strchr(q, ':');
-            if (!col) break;
-            if (k >= 1 && k < MF_NCLASS - 1 && atoi(col + 1) >= 256) want[k].fcap = atoi(col + 1);
-            q = strchr(col, ',');
-            if (q) q++;
-        }
-        if (memcmp(want, h_mf, sizeof(want)) != 0) {
-            memcpy(h_mf, want, sizeof(want));
-            NPB_CUDA(cudaMemcpyToSymbolAsync(c_mf, h_mf, sizeof(h_mf), 0, cudaMemcpyHostToDevice, s));
-        }
-    }
-    // test / A-B switches, read once per pass (the tests flip them between calls of one process)
+    // test switch, read once per pass (the tests flip it between calls of one process)
     const char *noleaf = getenv("NPB_GLS_NO_LEAF");   // every front through the general loop
     const int mf_flags = (noleaf && noleaf[0] == '1') ? 1 : 0;
-    const char *cap = getenv("NPB_GLS_CTAS_PER_SM");
-    const int env_cap = cap ? atoi(cap) : 0;
-    const char *var = getenv("NPB_GLS_VARIANT");
-    const int env_variant = var ? atoi(var) : 0;
     float main_ms = 0.f;
     static const char *cls_names[MF_NCLASS] = {"", "k2_gls_c1", "k2_gls_c2", "k2_gls_c3", "k2_gls_c4", "k2_gls_c5", "k2_gls_c6", "k2_gls_c7", "k2_gls_dense"};
     for (int k = 1; k < MF_NCLASS; k++) c->timings.erase(cls_names[k]);
@@ -1301,23 +1279,15 @@ int npb_k2_gls(npb_ctx *c, i64 lo, i64 hi)
         NpbTimer tk(c, cls_names[k]);
         int smem = (int)mf_smem_bytes(h_mf[k]);
         // resident warps per SM are bounded by shared memory; the launch bound follows it so that small
-        // stars trade registers for residency (24: 80 registers, 16: 128, 12: 168)
+        // stars trade registers for residency (16: 128 registers, 12: 168)
         int per_sm = (int)((227 * 1024) / (smem + 1024));
-        if (env_cap > 0 && per_sm > env_cap) per_sm = env_cap;
         if (per_sm > 32) per_sm = 32;
-        int variant = per_sm >= 16 ? 16 : 12;   // 24 (80 registers) spills the leaf fronts: only on request
-        if (env_variant == 12 || env_variant == 16 || env_variant == 24) variant = env_variant;
-        const int vregs = variant == 24 ? 80 : variant == 16 ? 128 : 168;
+        const int variant = per_sm >= 16 ? 16 : 12;
+        const int vregs = variant == 16 ? 128 : 168;
         if (per_sm > 65536 / (32 * vregs)) per_sm = 65536 / (32 * vregs);
         int grid = c->sm_count * per_sm;
         if (grid > count) grid = count;
         NPB_TRY(npb_ensure(&c->gls_ws, &c->gls_ws_cap, sizeof(double) * (size_t)grid * h_mf[k].acap * 2));
-#define MF_LAUNCH(V)                                                                                              \
-    do {                                                                                                          \
-        NPB_CUDA(cudaFuncSetAttribute(k_gls_mf<V>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));           \
-        k_gls_mf<V><<<grid, 32, smem, s>>>(a, list, count, counter, k, overflow, n_overflow, (double *)c->gls_ws, \
-                                           mf_flags);                                                             \
-    } while (0)
         // Team launch (the warps of an SM in one CTA, loosely in step, so that they share instruction fetches): pays
         // when the stars of the class are all alike - every node then runs the same instruction stream (structured
         // tets: -9 %) - and costs when they differ (mixed mesh: +20 %), so it is taken for the 168-register classes
@@ -1327,7 +1297,7 @@ int npb_k2_gls(npb_ctx *c, i64 lo, i64 hi)
         bool team_on = variant == 12 && per_sm == 12 && uniform_stars && count >= 12 * 64;
         int slack = 1, spins = 16;
         if (team) {
-            team_on = strcmp(team, "off") != 0 && variant != 24 && per_sm >= 2 && per_sm <= 32;
+            team_on = strcmp(team, "off") != 0 && per_sm >= 2 && per_sm <= 32;
             slack = atoi(team);
             const char *comma = strchr(team, ',');
             if (comma) spins = atoi(comma + 1);
@@ -1346,11 +1316,13 @@ int npb_k2_gls(npb_ctx *c, i64 lo, i64 hi)
                 k_gls_mf_team<12><<<grid, 32 * per_sm, tsmem, s>>>(a, list, count, counter, k, overflow, n_overflow,
                                                                   (double *)c->gls_ws, mf_flags, smem, slack, spins);
             }
-        } else
-        if (variant == 24) MF_LAUNCH(24);
-        else if (variant == 16) MF_LAUNCH(16);
-        else MF_LAUNCH(12);
-#undef MF_LAUNCH
+        } else if (variant == 16) {
+            NPB_CUDA(cudaFuncSetAttribute(k_gls_mf<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+            k_gls_mf<16><<<grid, 32, smem, s>>>(a, list, count, counter, k, overflow, n_overflow, (double *)c->gls_ws, mf_flags);
+        } else {
+            NPB_CUDA(cudaFuncSetAttribute(k_gls_mf<12>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+            k_gls_mf<12><<<grid, 32, smem, s>>>(a, list, count, counter, k, overflow, n_overflow, (double *)c->gls_ws, mf_flags);
+        }
         NPB_LAUNCH(c);
         NPB_CUDA(cudaGetLastError());
         tk.stop();

@@ -18,7 +18,6 @@
 // takes the general two-pass path (k2_idw_ls.cu + k3_emit.cu).
 #include <stdlib.h>
 #include "common.cuh"
-#include "tile_args.cuh"
 
 #define TILE_NB 64
 #define TILE_T 256
@@ -28,9 +27,6 @@
 #ifndef LS_ECAP
 #define LS_ECAP 1408
 #endif
-#ifndef LS_MINB
-#define LS_MINB 4   // 4 blocks of 46.8 KB fit an SM; 64 registers, no spills (5 would need <= 51)
-#endif
 #ifndef LS_ECAP_WIDE
 #define LS_ECAP_WIDE 1024
 #endif
@@ -38,12 +34,23 @@
 #define LS_NB_WIDE 128
 #endif
 #define IDW_EPS ((double)1.0000000036274937e-15f) /* float32(1e-15), idw.pyx:53 */
-#ifndef IDW_DEFAULT_VARIANT
-#define IDW_DEFAULT_VARIANT 0
-#endif
-#ifndef LS_DEFAULT_VARIANT
-#define LS_DEFAULT_VARIANT 1   // measured on B200 (tools/tile_sweep.py): LS 0.39 -> 0.52 (50M tets), 0.42 -> 0.50 (hex 200^3)
-#endif
+
+struct TileArgs {
+    const int32_t *esup_ptr, *esup;
+    const uint8_t *bpoint, *nflag;
+    const double *coords, *cent;
+    const int32_t *indptr;
+    int32_t *indices;
+    double *data;
+    int *zero_counter;
+    double *neumann;
+    double *wbuf;        // two-pass mode: values go to wbuf (esup-indexed from wbase) and rowcnt[p] = surviving entries
+    int32_t *rowcnt;
+    i64 wbase;
+    i64 p_lo, p_hi;      // node range of this launch
+    int nb, dim;
+    int direct;          // 1: write the CSR at indptr[] positions and count exact zeros; 0: two-pass mode
+};
 
 // rowcnt[p] = entries node p will emit if no weight is an exact zero; neumann[p] = 0
 __global__ void k_row_plan(const int32_t *__restrict__ esup_ptr, const uint8_t *__restrict__ bpoint,
@@ -62,8 +69,8 @@ __global__ void k_row_plan(const int32_t *__restrict__ esup_ptr, const uint8_t *
 }
 
 
-// MLPB = centroid loads batched per thread in phase A (0: the plain per-entry loop); MINB = resident CTAs asked for
-template <int NBCAP, int MINB, int MLPB>
+// MINB = resident CTAs asked for
+template <int NBCAP, int MINB>
 __global__ void __launch_bounds__(TILE_T, MINB) k_idw_tile(TileArgs a)
 {
     __shared__ double s_r[IDW_ECAP + NBCAP];
@@ -92,70 +99,25 @@ __global__ void __launch_bounds__(TILE_T, MINB) k_idw_tile(TileArgs a)
         if (tid < nb)
             for (int k = s_ptr[tid] - eb; k < s_ptr[tid + 1] - eb; k++) s_rid[k] = (unsigned char)tid;
         __syncthreads();
-        // phase A: one thread per esup entry.  Memory-level parallelism first: the ids of all of this thread's
-        // entries are fetched with independent loads, then the centroids in batches of MLP_B entries (9 loads in
-        // flight per thread), so a tile costs ~3 dependent global round trips instead of 2 per entry
-        if constexpr (MLPB == 0) {
-            for (int i = tid; i < ne; i += TILE_T) {
-                int node = s_rid[i];
-                if (!s_proc[node]) continue;
-                int e = a.esup[eb + i];
-                s_e[i] = e;
-                const double *cc = a.cent + (i64)e * NPB_CSTRIDE;
-                double d0 = __dsub_rn(s_x[3 * node], cc[0]);
-                double dist = __dadd_rn(0.0, __dmul_rn(d0, d0));
-                if (a.dim > 1) {
-                    double d1 = __dsub_rn(s_x[3 * node + 1], cc[1]);
-                    dist = __dadd_rn(dist, __dmul_rn(d1, d1));
-                }
-                if (a.dim > 2) {
-                    double d2 = __dsub_rn(s_x[3 * node + 2], cc[2]);
-                    dist = __dadd_rn(dist, __dmul_rn(d2, d2));
-                }
-                s_r[i + node] = (dist <= IDW_EPS) ? -1.0 : __ddiv_rn(1.0, __dsqrt_rn(dist));
+        // phase A: one thread per esup entry
+        for (int i = tid; i < ne; i += TILE_T) {
+            int node = s_rid[i];
+            if (!s_proc[node]) continue;
+            int e = a.esup[eb + i];
+            s_e[i] = e;
+            const double *cc = a.cent + (i64)e * NPB_CSTRIDE;
+            double d0 = __dsub_rn(s_x[3 * node], cc[0]);
+            double dist = __dadd_rn(0.0, __dmul_rn(d0, d0));
+            if (a.dim > 1) {
+                double d1 = __dsub_rn(s_x[3 * node + 1], cc[1]);
+                dist = __dadd_rn(dist, __dmul_rn(d1, d1));
             }
-        } else {
-            constexpr int KMAX = (IDW_ECAP + TILE_T - 1) / TILE_T;
-            constexpr int MLP_B = MLPB == 0 ? 1 : MLPB;
-            int ee[KMAX];
-#pragma unroll
-            for (int u = 0; u < KMAX; u++) {
-                const int i = tid + u * TILE_T;
-                ee[u] = (i < ne) ? a.esup[eb + i] : -1;
+            if (a.dim > 2) {
+                double d2 = __dsub_rn(s_x[3 * node + 2], cc[2]);
+                dist = __dadd_rn(dist, __dmul_rn(d2, d2));
             }
-#pragma unroll
-            for (int u0 = 0; u0 < KMAX; u0 += MLP_B) {
-                double c[MLP_B][3];
-#pragma unroll
-                for (int v = 0; v < MLP_B; v++) {
-                    const int u = u0 + v;
-                    if (u < KMAX && ee[u >= KMAX ? 0 : u] >= 0) {
-                        const double *cc = a.cent + (i64)ee[u >= KMAX ? 0 : u] * NPB_CSTRIDE;
-                        c[v][0] = cc[0]; c[v][1] = cc[1]; c[v][2] = cc[2];
-                    }
-                }
-#pragma unroll
-                for (int v = 0; v < MLP_B; v++) {
-                    const int u = u0 + v;
-                    if (u >= KMAX || ee[u >= KMAX ? 0 : u] < 0) continue;
-                    const int i = tid + u * TILE_T;
-                    const int node = s_rid[i];
-                    s_e[i] = ee[u >= KMAX ? 0 : u];
-                    if (!s_proc[node]) continue;
-                    double d0 = __dsub_rn(s_x[3 * node], c[v][0]);
-                    double dist = __dadd_rn(0.0, __dmul_rn(d0, d0));
-                    if (a.dim > 1) {
-                        double d1 = __dsub_rn(s_x[3 * node + 1], c[v][1]);
-                        dist = __dadd_rn(dist, __dmul_rn(d1, d1));
-                    }
-                    if (a.dim > 2) {
-                        double d2 = __dsub_rn(s_x[3 * node + 2], c[v][2]);
-                        dist = __dadd_rn(dist, __dmul_rn(d2, d2));
-                    }
-                    // coincident centroid (idw.pyx:69): marked with -1 (a reciprocal distance is never negative)
-                    s_r[i + node] = (dist <= IDW_EPS) ? -1.0 : __ddiv_rn(1.0, __dsqrt_rn(dist));
-                }
-            }
+            // coincident centroid (idw.pyx:69): marked with -1 (a reciprocal distance is never negative)
+            s_r[i + node] = (dist <= IDW_EPS) ? -1.0 : __ddiv_rn(1.0, __dsqrt_rn(dist));
         }
         __syncthreads();
         // phase B: one thread per node, sequential sum in esup order (idw.pyx:79)
@@ -214,7 +176,7 @@ __global__ void __launch_bounds__(TILE_T, MINB) k_idw_tile(TileArgs a)
 // NBCAP = node capacity of a tile: 64 for stars of >= 22 elements (tets); 128 (with 1024 entries) for small
 // stars such as the 8 hexes around a node, where 64 nodes would use a third of the entry capacity and leave
 // 3/4 of the threads idle in phase B (hex 200^3: 1.53 -> 1.08 ms)
-template <int ECAP, int NBCAP, int MINB, int MLPB>
+template <int ECAP, int NBCAP, int MINB>
 __global__ void __launch_bounds__(TILE_T, MINB) k_ls_tile(TileArgs a)
 {
     __shared__ double s_vx[ECAP + NBCAP], s_vy[ECAP + NBCAP], s_vz[ECAP + NBCAP];
@@ -243,50 +205,39 @@ __global__ void __launch_bounds__(TILE_T, MINB) k_ls_tile(TileArgs a)
         if (tid < nb)
             for (int k = s_ptr[tid] - eb; k < s_ptr[tid + 1] - eb; k++) s_rid[k] = (unsigned char)tid;
         __syncthreads();
-        // phase A: v = centroid - x_v per entry (ls.pyx:65-67); ids first, then the centroids in batches (see k_idw_tile)
-        if constexpr (MLPB == 0) {
-            for (int i = tid; i < ne; i += TILE_T) {
-                int node = s_rid[i];
-                if (!s_proc[node]) continue;
-                int e = a.esup[eb + i];
-                s_e[i] = e;
-                const double *cc = a.cent + (i64)e * NPB_CSTRIDE;
-                s_vx[i + node] = S2(cc[0], s_x[3 * node]);
-                s_vy[i + node] = S2(cc[1], s_x[3 * node + 1]);
-                s_vz[i + node] = S2(cc[2], s_x[3 * node + 2]);
-            }
-        } else {
-            constexpr int KMAX = (ECAP + TILE_T - 1) / TILE_T;
-            constexpr int MLP_B = MLPB == 0 ? 1 : MLPB;
-            int ee[KMAX];
+        // phase A: v = centroid - x_v per entry (ls.pyx:65-67).  Memory-level parallelism first: the ids of all of
+        // this thread's entries are fetched with independent loads, then the centroids in batches of MLP_B entries,
+        // so a tile costs ~3 dependent global round trips instead of 2 per entry
+        constexpr int KMAX = (ECAP + TILE_T - 1) / TILE_T;
+        constexpr int MLP_B = 2;
+        int ee[KMAX];
 #pragma unroll
-            for (int u = 0; u < KMAX; u++) {
+        for (int u = 0; u < KMAX; u++) {
+            const int i = tid + u * TILE_T;
+            ee[u] = (i < ne) ? a.esup[eb + i] : -1;
+        }
+#pragma unroll
+        for (int u0 = 0; u0 < KMAX; u0 += MLP_B) {
+            double c[MLP_B][3];
+#pragma unroll
+            for (int v = 0; v < MLP_B; v++) {
+                const int u = u0 + v;
+                if (u < KMAX && ee[u >= KMAX ? 0 : u] >= 0) {
+                    const double *cc = a.cent + (i64)ee[u >= KMAX ? 0 : u] * NPB_CSTRIDE;
+                    c[v][0] = cc[0]; c[v][1] = cc[1]; c[v][2] = cc[2];
+                }
+            }
+#pragma unroll
+            for (int v = 0; v < MLP_B; v++) {
+                const int u = u0 + v;
+                if (u >= KMAX || ee[u >= KMAX ? 0 : u] < 0) continue;
                 const int i = tid + u * TILE_T;
-                ee[u] = (i < ne) ? a.esup[eb + i] : -1;
-            }
-#pragma unroll
-            for (int u0 = 0; u0 < KMAX; u0 += MLP_B) {
-                double c[MLP_B][3];
-#pragma unroll
-                for (int v = 0; v < MLP_B; v++) {
-                    const int u = u0 + v;
-                    if (u < KMAX && ee[u >= KMAX ? 0 : u] >= 0) {
-                        const double *cc = a.cent + (i64)ee[u >= KMAX ? 0 : u] * NPB_CSTRIDE;
-                        c[v][0] = cc[0]; c[v][1] = cc[1]; c[v][2] = cc[2];
-                    }
-                }
-#pragma unroll
-                for (int v = 0; v < MLP_B; v++) {
-                    const int u = u0 + v;
-                    if (u >= KMAX || ee[u >= KMAX ? 0 : u] < 0) continue;
-                    const int i = tid + u * TILE_T;
-                    const int node = s_rid[i];
-                    s_e[i] = ee[u >= KMAX ? 0 : u];
-                    if (!s_proc[node]) continue;
-                    s_vx[i + node] = S2(c[v][0], s_x[3 * node]);
-                    s_vy[i + node] = S2(c[v][1], s_x[3 * node + 1]);
-                    s_vz[i + node] = S2(c[v][2], s_x[3 * node + 2]);
-                }
+                const int node = s_rid[i];
+                s_e[i] = ee[u >= KMAX ? 0 : u];
+                if (!s_proc[node]) continue;
+                s_vx[i + node] = S2(c[v][0], s_x[3 * node]);
+                s_vy[i + node] = S2(c[v][1], s_x[3 * node + 1]);
+                s_vz[i + node] = S2(c[v][2], s_x[3 * node + 2]);
             }
         }
         __syncthreads();
@@ -370,21 +321,19 @@ static int tile_nb(npb_ctx *c, int method)
     if (c->mx_epp <= 0) return 0;
     const char *force = getenv("NPB_FORCE_SIMPLE_IDW_LS");   // tests: exercise the thread-per-node kernels
     if (force && force[0] == '1') return 0;
-    const char *nowide = getenv("NPB_TILE_NO_WIDE");          // A/B timing: 64-node tiles only
-    const bool wide_ok = !(nowide && nowide[0] == '1');
     if (method == NPB_METHOD_IDW) {   // measured: 192-node IDW tiles are 25 % slower than 64-node ones on hex meshes
         int nb = IDW_ECAP / c->mx_epp;
         return nb > TILE_NB ? TILE_NB : nb;
     }
     int nb = LS_ECAP / c->mx_epp;
-    if (nb > TILE_NB && wide_ok) {
+    if (nb > TILE_NB) {
         int nw = LS_ECAP_WIDE / c->mx_epp;
         return nw > LS_NB_WIDE ? LS_NB_WIDE : nw;
     }
     return nb > TILE_NB ? TILE_NB : nb;
 }
 
-static void tile_args(npb_ctx *c, TileArgs &a, int method, i64 lo, i64 hi, int direct)
+static void tile_params(npb_ctx *c, TileArgs &a, int method, i64 lo, i64 hi, int direct)
 {
     a.esup_ptr = c->esup_ptr; a.esup = c->esup; a.bpoint = c->bpoint; a.nflag = c->nflag; a.coords = c->coords;
     a.cent = c->centroids; a.indptr = c->indptr; a.indices = c->indices; a.data = c->data;
@@ -398,37 +347,15 @@ static int tile_launch(npb_ctx *c, const TileArgs &a, int method)
     int grid = (int)(ntiles < (i64)c->sm_count * 8 ? ntiles : (i64)c->sm_count * 8);
     if (grid < 1) return NPB_OK;
     NpbTimer tm(c, "k2_main");
-    int piped = 0;
-    NPB_TRY(npb_tile_pipe_launch(c, a, method, &piped));
-    // NPB_TILE_VARIANT=<digit for IDW><digit for LS> picks among the compiled (resident CTAs, load batch) variants for
-    // A/B timing; the defaults are the measured best
-    const char *tv = getenv("NPB_TILE_VARIANT");
-    const int vi = (tv && tv[0] >= '0' && tv[0] <= '9') ? tv[0] - '0' : IDW_DEFAULT_VARIANT;
-    const int vl = (tv && tv[0] && tv[1] >= '0' && tv[1] <= '9') ? tv[1] - '0' : LS_DEFAULT_VARIANT;
-    if (piped) {
-    } else if (method == NPB_METHOD_IDW) {
-        switch (vi) {
-        case 1: k_idw_tile<TILE_NB, 7, 2><<<grid, TILE_T, 0, c->stream>>>(a); break;
-        case 2: k_idw_tile<TILE_NB, 6, 2><<<grid, TILE_T, 0, c->stream>>>(a); break;
-        case 3: k_idw_tile<TILE_NB, 5, 3><<<grid, TILE_T, 0, c->stream>>>(a); break;
-        case 4: k_idw_tile<TILE_NB, 4, 6><<<grid, TILE_T, 0, c->stream>>>(a); break;
-        default: k_idw_tile<TILE_NB, 7, 0><<<grid, TILE_T, 0, c->stream>>>(a); break;
-        }
-    } else if (a.nb > TILE_NB) {
-        switch (vl) {
-        case 1: k_ls_tile<LS_ECAP_WIDE, LS_NB_WIDE, 4, 2><<<grid, TILE_T, 0, c->stream>>>(a); break;
-        case 2: k_ls_tile<LS_ECAP_WIDE, LS_NB_WIDE, 4, 4><<<grid, TILE_T, 0, c->stream>>>(a); break;
-        case 3: k_ls_tile<LS_ECAP_WIDE, LS_NB_WIDE, 3, 4><<<grid, TILE_T, 0, c->stream>>>(a); break;
-        default: k_ls_tile<LS_ECAP_WIDE, LS_NB_WIDE, 4, 0><<<grid, TILE_T, 0, c->stream>>>(a); break;
-        }
-    } else {
-        switch (vl) {
-        case 1: k_ls_tile<LS_ECAP, TILE_NB, 4, 2><<<grid, TILE_T, 0, c->stream>>>(a); break;
-        case 2: k_ls_tile<LS_ECAP, TILE_NB, 4, 3><<<grid, TILE_T, 0, c->stream>>>(a); break;
-        case 3: k_ls_tile<LS_ECAP, TILE_NB, 3, 6><<<grid, TILE_T, 0, c->stream>>>(a); break;
-        default: k_ls_tile<LS_ECAP, TILE_NB, 4, 0><<<grid, TILE_T, 0, c->stream>>>(a); break;
-        }
-    }
+    // LS loads the centroids in batches (k_ls_tile phase A): 0.39 -> 0.52 of the HBM roofline on 50M tets, 0.42 -> 0.50
+    // on hex 200^3 against per-entry loads, which stay the faster choice for IDW (B200, DESIGN.md K2/K3).  LS asks for 4
+    // resident CTAs: 4 of 46.8 KB fit an SM; 64 registers, no spills (5 would need <= 51)
+    if (method == NPB_METHOD_IDW)
+        k_idw_tile<TILE_NB, 7><<<grid, TILE_T, 0, c->stream>>>(a);
+    else if (a.nb > TILE_NB)
+        k_ls_tile<LS_ECAP_WIDE, LS_NB_WIDE, 4><<<grid, TILE_T, 0, c->stream>>>(a);
+    else
+        k_ls_tile<LS_ECAP, TILE_NB, 4><<<grid, TILE_T, 0, c->stream>>>(a);
     NPB_LAUNCH(c);
     NPB_CUDA(cudaGetLastError());
     tm.stop_lazy();     // no host synchronisation between the tile kernel and whatever follows it on the stream
@@ -444,7 +371,7 @@ int npb_k2_idw_ls_tiles(npb_ctx *c, int method, i64 lo, i64 hi, int *used)
     *used = 1;
     if (hi <= lo) return NPB_OK;
     TileArgs a;
-    tile_args(c, a, method, lo, hi, 0);
+    tile_params(c, a, method, lo, hi, 0);
     return tile_launch(c, a, method);
 }
 
@@ -457,7 +384,7 @@ int npb_k2_idw_ls_direct(npb_ctx *c, int method, i64 lo, i64 hi, int *used)
     *used = 1;
     if (hi <= lo) return NPB_OK;
     TileArgs a;
-    tile_args(c, a, method, lo, hi, 1);
+    tile_params(c, a, method, lo, hi, 1);
     return tile_launch(c, a, method);
 }
 
@@ -479,7 +406,7 @@ int npb_k2_idw_ls_fused(npb_ctx *c, int method, int *used)
     NPB_CUDA(cudaStreamSynchronize(s));
     NPB_TRY(npb_ensure_out(c, (size_t)total));
     TileArgs a;
-    tile_args(c, a, method, 0, np, 1);
+    tile_params(c, a, method, 0, np, 1);
     NPB_TRY(tile_launch(c, a, method));
     int zeros = 0;
     NPB_CUDA(cudaMemcpyAsync(&zeros, zero_counter, sizeof(int), cudaMemcpyDeviceToHost, s));

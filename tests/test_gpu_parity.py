@@ -412,17 +412,14 @@ def test_out_of_range_node_ids_are_rejected_before_any_scatter():
     assert W.nnz > 0
 
 
-@pytest.mark.parametrize("shape", ["A", "B", "C", "D"])
-def test_pipelined_tile_kernels_bit_exact(shape, monkeypatch):
-    """The software-pipelined IDW / LS tile kernels (TMA bulk copies + cp.async gather, k2_tile_pipe.cu; opt-in with
-    NPB_TILE_PIPE) give bit-for-bit the oracle's values in every tile shape, over whole meshes and over the node
-    chunks of the pipeline (tiles then start at arbitrary nodes: unaligned bulk-copy sources)."""
+def test_tile_kernels_bit_exact():
+    """The IDW / LS tile kernels (k2_idw_ls_tile.cu) give bit-for-bit the oracle's values, over whole meshes and over
+    the node chunks of the pipeline (tiles then start at arbitrary nodes), on 64-node and wide 128-node LS tiles."""
     import ninpol_b200
     import oracle
     from ninpol_b200 import meshgen
-    monkeypatch.setenv("NPB_TILE_PIPE", shape)
-    for kind, n, kw in (("tet", 14, {}), ("hex", 20, {"perturb": 0.2}), ("mixed", 12, {"a": 3, "b": 6}), ("tet", 9, {"scramble": True}),
-                        ("tri2d", 12, {})):
+    for kind, n, kw in (("tet", 14, {}), ("hex", 20, {}), ("hex", 20, {"perturb": 0.2}), ("mixed", 12, {"a": 3, "b": 6}),
+                        ("tet", 9, {"scramble": True}), ("tri2d", 12, {}), ("quad2d", 9, {"perturb": 0.2})):
         mesh = meshgen.make_case(kind, n, **kw)
         O = oracle.OracleInterpolator().load_mesh(mesh)
         for chunks in (1, 7):
@@ -452,22 +449,3 @@ def test_both_esuel_kernels_bit_exact(kind, n, kw, monkeypatch):
         I.load_mesh(mesh_obj=mesh)
         for name in ("esuel", "infael", "inpofa", "esuf", "esuf_ptr", "boundary_faces", "boundary_points", "fsup"):
             assert np.array_equal(np.asarray(getattr(I.grid, name)), getattr(O.grid, name)), (name, plain)
-
-
-@pytest.mark.parametrize("variant", ["11", "22", "33", "40"])
-def test_tile_kernel_variants_bit_exact(variant, monkeypatch):
-    """The load-batched variants of the plain IDW / LS tile kernels (NPB_TILE_VARIANT) are the same arithmetic."""
-    import ninpol_b200
-    import oracle
-    from ninpol_b200 import meshgen
-    monkeypatch.setenv("NPB_TILE_VARIANT", variant)
-    for kind, n, kw in (("tet", 14, {}), ("hex", 20, {}), ("mixed", 12, {"a": 3, "b": 6}), ("quad2d", 9, {"perturb": 0.2})):
-        mesh = meshgen.make_case(kind, n, **kw)
-        O = oracle.OracleInterpolator().load_mesh(mesh)
-        I = ninpol_b200.Interpolator()
-        I.load_mesh(mesh_obj=mesh)
-        for method in ("idw", "ls"):
-            W, nv = I.interpolate("u", method)
-            Wo, nvo = O.interpolate("u", method)
-            assert np.array_equal(W.indptr, Wo.indptr) and np.array_equal(W.indices, Wo.indices), (kind, method)
-            assert np.array_equal(W.data, Wo.data, equal_nan=True), (kind, method)

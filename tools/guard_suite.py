@@ -91,11 +91,6 @@ run("tet", n3, "gls-dense", env={"NPB_FORCE_GLS_DENSE": "1"}, methods=("gls",))
 run("tet", n3, "gls-no-leaf", env={"NPB_GLS_NO_LEAF": "1"}, methods=("gls",))
 run("tet", n3 + 4, "gls-team", env={"NPB_GLS_TEAM": "1,16"}, methods=("gls",))
 run("mixed", n3 + 2, "gls-team", env={"NPB_GLS_TEAM": "0,4"}, methods=("gls",))
-run("mixed", n3 + 2, "gls-small-front", env={"NPB_GLS_FCAP": "512"}, methods=("gls",))
-for shape in ("A", "B", "C", "D"):
-    run("tet", n3, "tile-pipe-" + shape, env={"NPB_TILE_PIPE": shape}, methods=("idw", "ls"))
-for v in ("0", "1", "2", "3"):
-    run("hex", n3, "tile-variant-" + v, env={"NPB_TILE_VARIANT": v}, methods=("idw", "ls"))
 run("hex", n3, "no-neumann", neumann_rate=0.0)
 plugin("tet", n3)
 print("guard suite done", flush=True)
