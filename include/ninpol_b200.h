@@ -156,6 +156,19 @@ int npb_interpolate_fetch(npb_ctx *ctx, int32_t *indptr, int32_t *indices, doubl
  * "d2h_apply" (and "k3_fill" when the rows still had to be written). */
 int npb_apply(npb_ctx *ctx, int method, const double *values, int64_t n_cols, double *out);
 
+/* K5 — the transposed product from the resident weights: adjoints / gradients through the nodal reconstruction,
+ * transposed matrix-free solves, least-squares fits of a cell field to nodal data (scipy: `W.T @ y`).
+ * out[e, c] = sum over the entries (p, e) of W in ascending p of data[j] * values[p, c], for c < n_cols, using the CSR
+ * of `method` that the last npb_interpolate_count / npb_interpolate_run left on the device.  Each sum starts at +0.0
+ * and every product and addition is rounded on its own: bit-identical to scipy's csc_matvec(s) on the view W.T.
+ * values [n_points, n_cols] and out [n_elems, n_cols]: float64, row-major, host memory (pageable or page-locked).
+ * NPB_ERR_STATE when no CSR of `method` is resident, exactly as npb_apply.  NPB_ERR_STATE when world > 1: a rank holds
+ * only its own rows, so the ordered sum of an element spans ranks; the transposed product is single-GPU.
+ * The first call on a CSR builds a map of every element's (node, CSR position) slots (8 * spe bytes per element); it
+ * is rebuilt whenever the CSR is rewritten or voided.  Timings: "h2d_adjoint" "adjoint_map" (0 when the map was
+ * reused) "adjoint" "d2h_adjoint" (and "k3_fill" when the rows still had to be written). */
+int npb_apply_transpose(npb_ctx *ctx, int method, const double *values, int64_t n_cols, double *out);
+
 /* The plug-in's own output, for callers that sit where Interpolator.prepare_interpolator sits
  * (interpolator.pyx:631-670): dense weights [n_points, MX_ELEMENTS_PER_POINT] (row stride
  * MX_ELEMENTS_PER_POINT, column k of row p <-> esup[esup_ptr[p] + k], untouched entries 0) and neumann_ws

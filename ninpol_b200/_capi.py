@@ -44,6 +44,7 @@ _SIGNATURES = {
                             + [ctypes.c_int64, _c_i64p, ctypes.POINTER(ctypes.c_int)]),
     "npb_interpolate_streamed": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int, ctypes.c_int] + [ctypes.c_void_p] * 6 + [ctypes.c_int64, _c_i64p]),
     "npb_apply": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_int64, ctypes.c_void_p]),
+    "npb_apply_transpose": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_int64, ctypes.c_void_p]),
     "npb_timing": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_char_p, ctypes.POINTER(ctypes.c_double)]),
     "npb_launch_count": (ctypes.c_int, [ctypes.c_void_p, _c_i64p]),
     "npb_check_guards": (ctypes.c_int, [ctypes.c_void_p, _c_i64p, _c_i64p]),
@@ -246,6 +247,15 @@ class Context:
         k = 1 if values.ndim == 1 else int(values.shape[1])
         assert values.ndim in (1, 2) and out.ndim == values.ndim and out.shape[1:] == values.shape[1:]
         check(self.lib.npb_apply(self.handle, METHOD_IDS[method], _ptr(values), k, _ptr(out)))
+
+    def apply_transpose(self, method, values, out):
+        """out[:] = W.T @ values with the CSR of `method` resident on the device (npb_apply_transpose).  values
+        [n_points, k] and out [n_elems, k]: float64, C-contiguous (1-D: k = 1).  One GPU only."""
+        assert values.dtype == np.float64 and out.dtype == np.float64
+        assert values.flags.c_contiguous and out.flags.c_contiguous
+        k = 1 if values.ndim == 1 else int(values.shape[1])
+        assert values.ndim in (1, 2) and out.ndim == values.ndim and out.shape[1:] == values.shape[1:]
+        check(self.lib.npb_apply_transpose(self.handle, METHOD_IDS[method], _ptr(values), k, _ptr(out)))
 
     # --- measurement ---
     def timing(self, name):

@@ -292,6 +292,7 @@ static void free_mesh(npb_ctx *c)
     c->fused_failed[0] = c->fused_failed[1] = false;
     c->mesh_loaded = false;
     c->counted = false;
+    c->csr_gen++;
     c->plan_kind = 0;
     c->plan_chunks = 0;
     c->chunk_node.clear();
@@ -366,6 +367,7 @@ extern "C" int npb_destroy(npb_ctx *c)
     if (c->gls_ws) { npb_guard_forget(c->gls_ws); cudaFree(c->gls_ws); }
     if (c->apply_x) { npb_guard_forget(c->apply_x); cudaFree(c->apply_x); }
     if (c->apply_y) { npb_guard_forget(c->apply_y); cudaFree(c->apply_y); }
+    if (c->tmap) { npb_guard_forget(c->tmap); cudaFree(c->tmap); }
     if (c->counters) cudaFree(c->counters);
     if (c->h_small) cudaFreeHost(c->h_small);
     for (int i = 0; i < 2; i++) {
@@ -409,6 +411,7 @@ static int refresh_range(npb_ctx *c)
     c->wbase = b[0];
     c->wlen = (i64)b[1] - b[0];
     c->counted = false;
+    c->csr_gen++;
     c->plan_chunks = 0;   // chunk boundaries follow the rank bounds
     c->apply_range_ok = false;
     return NPB_OK;
@@ -443,6 +446,7 @@ extern "C" int npb_set_gather(npb_ctx *c, int mode)
     }
     c->gather_mode = mode;
     c->counted = false;
+    c->csr_gen++;
     return NPB_OK;
 }
 
@@ -660,6 +664,7 @@ extern "C" int npb_set_cell_field(npb_ctx *c, const char *name, const double *da
     }
     NPB_CUDA(cudaStreamSynchronize(c->stream));
     c->counted = false;
+    c->csr_gen++;
     c->plan_failed[NPB_METHOD_GLS] = false;
     return NPB_OK;
 }
@@ -692,6 +697,7 @@ extern "C" int npb_set_cell_field_range(npb_ctx *c, const char *name, const doub
     }
     NPB_CUDA(cudaStreamSynchronize(c->stream));
     c->counted = false;
+    c->csr_gen++;
     c->plan_failed[NPB_METHOD_GLS] = false;
     return NPB_OK;
 }
@@ -749,6 +755,7 @@ extern "C" int npb_set_point_flags(npb_ctx *c, const int64_t *flag, int64_t n_po
     NPB_TRY(read_flag_checksum(c));
     c->have_flags = true;
     c->counted = false;
+    c->csr_gen++;
     c->plan_kind = 0;     // row lengths depend on the flags
     c->plan_failed[0] = c->plan_failed[1] = c->plan_failed[2] = false;
     c->fused_failed[0] = c->fused_failed[1] = false;
@@ -799,6 +806,7 @@ extern "C" int npb_set_point_flags_f64(npb_ctx *c, const double *flag, int64_t n
     NPB_TRY(read_flag_checksum(c));
     c->have_flags = true;
     c->counted = false;
+    c->csr_gen++;
     c->plan_kind = 0;     // row lengths depend on the flags
     c->plan_failed[0] = c->plan_failed[1] = c->plan_failed[2] = false;
     c->fused_failed[0] = c->fused_failed[1] = false;
@@ -840,6 +848,7 @@ extern "C" int npb_set_point_flags_f64_range(npb_ctx *c, const double *flag_slic
     *checksum = (i64)(h >> 1);
     if (*checksum != c->flags_checksum) {   // the flags changed somewhere: this device's copy is no longer trustworthy
         c->counted = false;
+        c->csr_gen++;
         c->plan_kind = 0;
     }
     return NPB_OK;
@@ -870,6 +879,7 @@ extern "C" int npb_interpolate_count(npb_ctx *c, int method, int64_t *nnz)
     NPB_CUDA(cudaSetDevice(c->device));
     cudaStream_t s = c->stream;
     c->filled = false;
+    c->csr_gen++;
     c->gathered = false;
     c->plan_kind = 0;     // this path rewrites indptr / neumann
     if (method != NPB_METHOD_GLS && !c->fused_failed[method]) {
@@ -885,6 +895,7 @@ extern "C" int npb_interpolate_count(npb_ctx *c, int method, int64_t *nnz)
             c->method = method;
             c->counted = true;
             c->filled = true;
+            c->csr_gen++;
             c->nnz_ret = c->nnz;
             c->blk_off = 0;
             *nnz = c->nnz;
@@ -934,6 +945,7 @@ extern "C" int npb_interpolate_count(npb_ctx *c, int method, int64_t *nnz)
     }
     c->method = method;
     c->counted = true;
+    c->csr_gen++;
     *nnz = c->nnz_ret;
     return NPB_OK;
 }
@@ -988,6 +1000,7 @@ extern "C" int npb_interpolate_fetch(npb_ctx *c, int32_t *indptr, int32_t *indic
         NPB_TRY(npb_k3_fill(c, c->lo, c->hi));
         tm.stop();
         c->filled = true;
+        c->csr_gen++;
     }
     const bool host_gather = c->world > 1 && c->gather_mode == NPB_GATHER_HOST;
     if (c->world > 1 && !host_gather && !c->gathered) {
@@ -1034,8 +1047,21 @@ extern "C" int npb_interpolate_fetch(npb_ctx *c, int32_t *indptr, int32_t *indic
 }
 
 // ------------------------------------------------------------------------------------------------
-// K5 — nodal values W @ values from the CSR left on the device by the last count / run
+// K5 — nodal values W @ values (and W.T @ values) from the CSR left on the device by the last count / run
 // ------------------------------------------------------------------------------------------------
+// the two-pass count (exact-zero fallback, or world > 1) leaves the rows unwritten: write them before a product
+static int fill_rows_for_apply(npb_ctx *c)
+{
+    if (c->filled) return NPB_OK;
+    NPB_TRY(npb_ensure_out(c, (size_t)c->nnz));
+    NpbTimer tm(c, "k3_fill");
+    NPB_TRY(npb_k3_fill(c, c->lo, c->hi));
+    tm.stop_lazy();
+    c->filled = true;
+    c->csr_gen++;
+    return NPB_OK;
+}
+
 extern "C" int npb_apply(npb_ctx *c, int method, const double *values, int64_t n_cols, double *out)
 {
     if (!c || n_cols < 0 || (n_cols > 0 && (!values || !out))) return NPB_ERR_ARG;
@@ -1046,13 +1072,7 @@ extern "C" int npb_apply(npb_ctx *c, int method, const double *values, int64_t n
     }
     if (n_cols == 0) return NPB_OK;
     NPB_CUDA(cudaSetDevice(c->device));
-    if (!c->filled) {   // the two-pass count (exact-zero fallback, or world > 1) left the rows unwritten
-        NPB_TRY(npb_ensure_out(c, (size_t)c->nnz));
-        NpbTimer tm(c, "k3_fill");
-        NPB_TRY(npb_k3_fill(c, c->lo, c->hi));
-        tm.stop_lazy();
-        c->filled = true;
-    }
+    NPB_TRY(fill_rows_for_apply(c));
     // this rank's nodes read the values of the elements in their esup rows only: upload that slice
     i64 first = 0, last = c->n_elems - 1;
     if (c->world > 1) {
@@ -1087,6 +1107,53 @@ extern "C" int npb_apply(npb_ctx *c, int method, const double *values, int64_t n
     {
         NpbTimer tm(c, "d2h_apply");
         NPB_TRY(npb_d2h(c, out, c->apply_y, sizeof(double) * (size_t)(c->n_points * n_cols)));
+        tm.stop();
+    }
+    NPB_CUDA(cudaStreamSynchronize(c->stream));
+    return NPB_OK;
+}
+
+// W.T @ values: one GPU only.  A rank holds only its own rows, so the ascending-node sum of an element would span ranks.
+extern "C" int npb_apply_transpose(npb_ctx *c, int method, const double *values, int64_t n_cols, double *out)
+{
+    if (!c || n_cols < 0 || (n_cols > 0 && (!values || !out))) return NPB_ERR_ARG;
+    if (c->world > 1) {
+        npb_set_error("npb_apply_transpose: the transposed product is single-GPU (world is %d): every rank holds only its "
+                      "own rows of W, and the ascending-node sum of an element spans ranks", c->world);
+        return NPB_ERR_STATE;
+    }
+    if (!c->counted || c->method != method) {
+        npb_set_error("npb_apply_transpose: no weights of method %d are resident (run npb_interpolate_count or "
+                      "npb_interpolate_run for the current inputs first)", method);
+        return NPB_ERR_STATE;
+    }
+    if (n_cols == 0) return NPB_OK;
+    NPB_CUDA(cudaSetDevice(c->device));
+    NPB_TRY(fill_rows_for_apply(c));
+    if (c->tmap_gen != c->csr_gen) {
+        NPB_TRY(npb_ensure((void **)&c->tmap, &c->tmap_cap, sizeof(int2) * (size_t)(c->n_elems * c->spe)));
+        NpbTimer tm(c, "adjoint_map");
+        NPB_TRY(npb_k5_tmap(c, c->tmap));
+        tm.stop();   // synchronous: a reused map below records 0 with no pending timer left to overwrite it
+        c->tmap_gen = c->csr_gen;
+    } else {
+        c->timings["adjoint_map"] = 0.f;
+    }
+    NPB_TRY(npb_ensure((void **)&c->apply_y, &c->apply_y_cap, sizeof(double) * (size_t)(c->n_points * n_cols)));
+    NPB_TRY(npb_ensure((void **)&c->apply_x, &c->apply_x_cap, sizeof(double) * (size_t)(c->n_elems * n_cols)));
+    {
+        NpbTimer tm(c, "h2d_adjoint");
+        NPB_TRY(npb_h2d(c, c->apply_y, values, sizeof(double) * (size_t)(c->n_points * n_cols)));
+        tm.stop_lazy();
+    }
+    {
+        NpbTimer tm(c, "adjoint");
+        NPB_TRY(npb_k5_apply_t(c, c->tmap, c->apply_y, n_cols, c->apply_x));
+        tm.stop_lazy();
+    }
+    {
+        NpbTimer tm(c, "d2h_adjoint");
+        NPB_TRY(npb_d2h(c, out, c->apply_x, sizeof(double) * (size_t)(c->n_elems * n_cols)));
         tm.stop();
     }
     NPB_CUDA(cudaStreamSynchronize(c->stream));
@@ -1137,6 +1204,7 @@ extern "C" int npb_interpolate_dense(npb_ctx *c, int method, double *weights, do
     cudaStream_t s = c->stream;
     c->counted = false;
     c->filled = false;
+    c->csr_gen++;
     NPB_TRY(npb_ensure((void **)&c->wbuf, &c->wbuf_cap, sizeof(double) * (size_t)(c->wlen > 0 ? c->wlen : 1)));
     if (method == NPB_METHOD_GLS)
         NPB_TRY(npb_k2_gls(c, c->lo, c->hi));

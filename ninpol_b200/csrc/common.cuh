@@ -113,6 +113,9 @@ struct npb_ctx {
     bool counted = false;
     bool fused_failed[2] = {false, false};   // per method: the single-pass emit met an exact zero for the current inputs
     bool filled = false;         // indices / data already hold the CSR (fused path, or k3_fill done)
+    // bumped at every write or voiding of the CSR rows (each counted / filled transition): what is derived from the CSR
+    // (the transposed map below) records the generation it was built from and is rebuilt when it differs
+    unsigned long long csr_gen = 1;
     i64 nnz = 0;
     i64 nnz_ret = 0, blk_off = 0;   // what count / fetch hand out: all of it, or this rank's row block (gather to root)
     int gather_mode = 0;            // NPB_GATHER_ALL / NPB_GATHER_ROOT
@@ -148,11 +151,17 @@ struct npb_ctx {
     std::vector<i64> chunk_node, chunk_nz;   // [world * K + 1] node / nnz boundaries of every rank's chunks
     std::vector<i64> chunk_efirst, chunk_elast;   // [K] element range this rank's chunk k reads (empty: not computed yet)
     bool gathered = false;               // indices / data / neumann of ALL ranks are on this device (gather = all)
-    // npb_apply (k5_apply.cu): the values uploaded for this rank's rows and the result rows, [.., n_cols] row-major
+    // npb_apply (k5_apply.cu): the values uploaded for this rank's rows and the result rows, [.., n_cols] row-major.
+    // npb_apply_transpose uses the same two buffers by shape: apply_y holds its nodal input, apply_x its element output
     double *apply_x = nullptr, *apply_y = nullptr;
     size_t apply_x_cap = 0, apply_y_cap = 0;
     bool apply_range_ok = false;         // apply_first / apply_last hold npb_partition_elem_range for the current partition
     i64 apply_first = 0, apply_last = -1;
+    // npb_apply_transpose: [n_elems, spe] (node, CSR position) slots of every element, built from the CSR of generation
+    // tmap_gen (k5_tmap)
+    int2 *tmap = nullptr;
+    size_t tmap_cap = 0;
+    unsigned long long tmap_gen = 0;
 };
 
 // ---- helpers implemented in capi.cu ----
@@ -201,6 +210,8 @@ int npb_k4_gather_counts(npb_ctx *c);
 int npb_k4_gather_blocks(npb_ctx *c);
 int npb_k4_gather_rows(npb_ctx *c, double *rows, i64 n_cols);
 int npb_k5_apply(npb_ctx *c, i64 lo, i64 hi, const double *x, int64_t k, double *out);
+int npb_k5_tmap(npb_ctx *c, int2 *map);
+int npb_k5_apply_t(npb_ctx *c, const int2 *map, const double *y, int64_t k, double *out);
 int npb_export_array(npb_ctx *c, const char *name, void *out, i64 cap);
 // cudaMalloc'ed temporary that is freed when it goes out of scope (error returns included)
 struct NpbTmp {

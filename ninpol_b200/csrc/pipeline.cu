@@ -162,6 +162,7 @@ static int run_pipeline(npb_ctx *c, int method, int K, const double *perm_host, 
     if (gls) NPB_TRY(npb_ensure((void **)&c->wbuf, &c->wbuf_cap, sizeof(double) * (size_t)(c->wlen > 0 ? c->wlen : 1)));
     c->counted = false;
     c->filled = false;
+    c->csr_gen++;
     int *bad = c->counters + 45;   // [45] exact zeros (tile kernels), [46] row-count mismatches (planned emit)
     NPB_CUDA(cudaMemsetAsync(bad, 0, 2 * sizeof(int), s));
     cudaEvent_t ev_start = c->pipe_ev[3 * K], ev_side = c->pipe_ev[3 * K + 1];
@@ -315,6 +316,7 @@ static int run_pipeline(npb_ctx *c, int method, int K, const double *perm_host, 
     c->method = method;
     c->counted = true;     // a later npb_interpolate_fetch copies these very arrays
     c->filled = true;
+    c->csr_gen++;
     c->gathered = nccl_gather;
     return NPB_OK;
 }

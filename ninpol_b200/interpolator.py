@@ -7,6 +7,7 @@ Same constructor keywords, methods and attributes as the reference class
     I.load_mesh(mesh_obj=mesh)                       # or filename=... when meshio is installed
     W, neumann = I.interpolate("pressure", "gls")    # scipy CSR (n_nodes, n_elements), ndarray (n_nodes,)
     u_nodes = I.nodal_values("pressure", "gls")     # W @ u on the GPU, bit for bit; the weights stay resident
+    g_cells = I.nodal_adjoint("pressure", "gls", g_nodes)   # W.T @ g on the GPU (one GPU), same weights, bit for bit
     I.supported_methods                              # {"gls": ..., "idw": ..., "ls": ...}
 
 The host side only ingests the mesh object (vectorised numpy instead of the reference's per-item Python
@@ -636,8 +637,8 @@ class Interpolator:
 
     def invalidate_inputs(self):
         """Forget which per-variable inputs are resident on the device: the next interpolate() uploads
-        the flags (and, for GLS, permeability + diff_mag) again from host memory, and nodal_values() recomputes the
-        weights."""
+        the flags (and, for GLS, permeability + diff_mag) again from host memory, and nodal_values() / nodal_adjoint()
+        recompute the weights."""
         self._staged = None
         self._weights_key = None
 
@@ -819,19 +820,11 @@ class Interpolator:
             row = np.asarray(self._rows["cells"][self.variable_to_index["cells"][variable]], dtype=DTYPE_F)
             x = row[:n_elems * dim] if dim == 1 else row[:n_elems * dim].reshape(n_elems, dim)
         else:
-            if np.iscomplexobj(values):
-                raise TypeError("nodal_values: complex values are not supported; pass the real and imaginary parts "
-                                "as separate columns")
-            x = np.asarray(values, dtype=DTYPE_F)
-            if x.ndim not in (1, 2) or x.shape[0] != n_elems:
-                raise ValueError(f"nodal_values: values must have shape ({n_elems},) or ({n_elems}, k), got {x.shape}")
+            x = self._as_real_rows("nodal_values", values, n_elems)
         x = np.ascontiguousarray(x)
         if x.ndim == 2 and x.shape[1] == 0:
             return np.empty((n_points, 0), dtype=DTYPE_F)
-        key = (method, variable, self._data_version, self._mesh_serial)
-        reused = self._weights_key == key
-        if not reused:
-            self._compute_weights(variable, method, fetch=False)
+        reused = self._resident_weights(variable, method)
         out = self._out("nodal", n_points * (1 if x.ndim == 1 else x.shape[1]), DTYPE_F)
         out = out.reshape((n_points,) + x.shape[1:])
         self._ctx.apply(method, x, out)
@@ -839,3 +832,51 @@ class Interpolator:
         self.last_timings.update({"nodal_h2d_ms": t("h2d_apply"), "nodal_apply_ms": t("apply"),
                                   "nodal_d2h_ms": t("d2h_apply"), "nodal_weights_reused": reused})
         return out
+
+    def nodal_adjoint(self, variable, method, values):
+        """The transposed product `W.T @ values`, where W is the CSR `interpolate(variable, method)` returns, computed on
+        the GPU from the resident weights: bit-identical to scipy's product (NaN included).  It takes nodal values or
+        sensitivities back to the cells: gradients through the nodal reconstruction (d f(W u) / du = W.T df/dy),
+        transposed matrix-free solves, least-squares fits of a cell field to nodal data.  The weights are shared with
+        nodal_values(): alternating the two on unchanged inputs computes them once.
+
+        values: any real array of shape (n_points,) or (n_points, k), converted to float64 like scipy does.  Returns
+        float64 of shape (n_elems,) or (n_elems, k).  One GPU only: with several ranks it raises NotImplementedError,
+        since every rank holds only its own rows of W."""
+        self._check_call(variable, method)
+        if self.comm.world > 1:
+            raise NotImplementedError("nodal_adjoint: the transposed product is single-GPU; every rank holds only its "
+                                      "own rows of W")
+        g = self.grid
+        n_elems, n_points = g.n_elems, g.n_points
+        y = np.ascontiguousarray(self._as_real_rows("nodal_adjoint", values, n_points))
+        if y.ndim == 2 and y.shape[1] == 0:
+            return np.empty((n_elems, 0), dtype=DTYPE_F)
+        reused = self._resident_weights(variable, method)
+        out = self._out("adjoint", n_elems * (1 if y.ndim == 1 else y.shape[1]), DTYPE_F)
+        out = out.reshape((n_elems,) + y.shape[1:])
+        self._ctx.apply_transpose(method, y, out)
+        t = self._ctx.timing_or
+        self.last_timings.update({"adjoint_h2d_ms": t("h2d_adjoint"), "adjoint_map_ms": t("adjoint_map"),
+                                  "adjoint_apply_ms": t("adjoint"), "adjoint_d2h_ms": t("d2h_adjoint"),
+                                  "adjoint_weights_reused": reused})
+        return out
+
+    @staticmethod
+    def _as_real_rows(caller, values, n_rows):
+        """values as float64 of shape (n_rows,) or (n_rows, k), the operand checks of nodal_values / nodal_adjoint."""
+        if np.iscomplexobj(values):
+            raise TypeError(f"{caller}: complex values are not supported; pass the real and imaginary parts "
+                            "as separate columns")
+        x = np.asarray(values, dtype=DTYPE_F)
+        if x.ndim not in (1, 2) or x.shape[0] != n_rows:
+            raise ValueError(f"{caller}: values must have shape ({n_rows},) or ({n_rows}, k), got {x.shape}")
+        return x
+
+    def _resident_weights(self, variable, method):
+        """Makes the CSR of (method, variable) for the current inputs resident on the device, computing it only when
+        the resident one is not that; returns True when it was reused."""
+        reused = self._weights_key == (method, variable, self._data_version, self._mesh_serial)
+        if not reused:
+            self._compute_weights(variable, method, fetch=False)
+        return reused

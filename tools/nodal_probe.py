@@ -9,7 +9,15 @@ kernel has to move, 12 nnz + 4 (rows + 1) + 8k (elements read) + 8k rows, over t
 rate (npb_measure_copy_bw).  The working set (> 2 GB at C4) is far larger than the 126 MB L2, so every call reads HBM.
 For comparison: interpolate() + scipy's W @ u on the host, and the first nodal_values() call, which computes the
 weights.  The full results are checked bit for bit against W @ u.  The card's name, power limit and SM clock are read
-with nvidia-smi in the same run."""
+with nvidia-smi in the same run.
+
+    python tools/nodal_probe.py --adjoint [--out profiles/nodal_adjoint_probe.json] [--workloads ...] [--reps 7]
+
+The same for Interpolator.nodal_adjoint (W.T @ y) on the same workloads: the first call (weights and map computed by the
+adjoint itself) and the map build inside it, the median wall time on fresh values with weights and map resident split
+into H2D / kernel (npb_timing "adjoint") / D2H, the kernel's bytes, 8 spe n_elems (map) + 8 nnz (data) + 8k nnz (y
+gathers) + 8k n_elems (out), as a fraction of the copy rate (and the same with y counted once, 8k n_points), scipy's
+W.T @ y on the host, and bit-equality of the full results."""
 import argparse
 import json
 import os
@@ -129,12 +137,83 @@ def probe(name, reps, copy_gbs):
     return res
 
 
+def probe_adjoint(name, reps, copy_gbs):
+    kind, n, rate, method, desc = WORKLOADS[name]
+    t0 = time.perf_counter()
+    mesh = meshgen.make_case(kind, n, neumann_rate=rate)
+    spe = 4 if max(len(c.data[0]) for c in mesh.cells) <= 4 else 8
+    I = ninpol_b200.Interpolator()
+    I.load_mesh(mesh_obj=mesh)
+    g = I.grid
+    print(f"[{name}] mesh ready in {time.perf_counter() - t0:.1f} s: {g.n_elems} cells, {g.n_points} nodes", flush=True)
+    res = {"workload": desc, "method": method, "n_elems": int(g.n_elems), "n_points": int(g.n_points), "spe": spe}
+    rng = np.random.default_rng(5)
+
+    # the first call computes the weights (no CSR download) and builds the map; timed after one untimed warm-up
+    y_first = rng.standard_normal(g.n_points)
+    first, maps = [], []
+    for rep in range(1 + min(reps, 3)):
+        I.invalidate_inputs()
+        ms, z_first = wall(lambda: I.nodal_adjoint("u", method, y_first), I)
+        assert not I.last_timings["adjoint_weights_reused"]
+        if rep:
+            first.append(ms)
+            maps.append(I.last_timings["adjoint_map_ms"])
+    res["first_call_with_weights_ms_median"] = float(np.median(first))
+    res["map_build_ms_median"] = float(np.median(maps))
+
+    W, _ = I.interpolate("u", method)
+    res["bit_equal_first_call"] = same_bits(z_first, W.T @ y_first)
+    nnz = int(W.nnz)
+    res["nnz"] = nnz
+    for k in (1, 3):
+        ys = [rng.standard_normal(g.n_points) if k == 1 else rng.standard_normal((g.n_points, k)) for _ in range(2)]
+        walls, kern, h2d, d2h = [], [], [], []
+        for rep in range(reps + 2):        # the first call after interpolate() rebuilds the map: warm-up
+            y = ys[rep % 2] + rep          # fresh values every call (not timed)
+            ms, z = wall(lambda: I.nodal_adjoint("u", method, y), I)
+            assert I.last_timings["adjoint_weights_reused"]
+            if rep >= 2:
+                assert I.last_timings["adjoint_map_ms"] == 0.0
+                walls.append(ms)
+                kern.append(I.last_timings["adjoint_apply_ms"])
+                h2d.append(I.last_timings["adjoint_h2d_ms"])
+                d2h.append(I.last_timings["adjoint_d2h_ms"])
+        t1 = time.perf_counter()
+        want = W.T @ y
+        ms_host = (time.perf_counter() - t1) * 1e3
+        bytes_needed = 8 * spe * g.n_elems + 8 * nnz + 8 * k * nnz + 8 * k * g.n_elems
+        # each array once (the y gathers of one node repeat over its elements and mostly hit L2)
+        bytes_once = 8 * spe * g.n_elems + 8 * nnz + 8 * k * g.n_points + 8 * k * g.n_elems
+        kms = float(np.median(kern))
+        res[f"k{k}"] = {
+            "nodal_adjoint_wall_ms_median": float(np.median(walls)),
+            "adjoint_kernel_ms_median": kms,
+            "adjoint_kernel_ms_min": float(np.min(kern)),
+            "h2d_ms_median": float(np.median(h2d)),
+            "d2h_ms_median": float(np.median(d2h)),
+            "bytes_model": int(bytes_needed),
+            "adjoint_gbs": bytes_needed / (kms * 1e-3) / 1e9,
+            "fraction_of_copy_bw": bytes_needed / (kms * 1e-3) / (copy_gbs * 1e9),
+            "bytes_each_array_once": int(bytes_once),
+            "fraction_of_copy_bw_each_array_once": bytes_once / (kms * 1e-3) / (copy_gbs * 1e9),
+            "host_scipy_transposed_dot_ms": ms_host,
+            "bit_equal": same_bits(z, want),
+        }
+        print(f"[{name}] k={k}: {json.dumps(res[f'k{k}'])}", flush=True)
+    del W
+    return res
+
+
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument("--out", default=os.path.join("profiles", "nodal_probe.json"))
+    ap.add_argument("--adjoint", action="store_true", help="probe nodal_adjoint (W.T @ y) instead of nodal_values")
+    ap.add_argument("--out", default=None)
     ap.add_argument("--workloads", default="c4_gls,c3_idw")
     ap.add_argument("--reps", type=int, default=7)
     args = ap.parse_args()
+    if args.out is None:
+        args.out = os.path.join("profiles", "nodal_adjoint_probe.json" if args.adjoint else "nodal_probe.json")
     from ninpol_b200 import _capi
     ctx = _capi.Context(0)
     copy_gbs = ctx.measure_copy_bw(1 << 31)
@@ -144,13 +223,13 @@ def main():
     print(f"card {out['card']}; device copy {copy_gbs:.0f} GB/s", flush=True)
     ok = True
     for name in args.workloads.split(","):
-        r = probe(name, args.reps, copy_gbs)
+        r = (probe_adjoint if args.adjoint else probe)(name, args.reps, copy_gbs)
         out["results"][name] = r
         ok = ok and r["bit_equal_first_call"] and r["k1"]["bit_equal"] and r["k3"]["bit_equal"]
     os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
     with open(args.out, "w") as f:
         json.dump(out, f, indent=1)
-    print("nodal probe", "bit-equal" if ok else "MISMATCH", "->", args.out, flush=True)
+    print("nodal adjoint probe" if args.adjoint else "nodal probe", "bit-equal" if ok else "MISMATCH", "->", args.out, flush=True)
     sys.exit(0 if ok else 1)
 
 
